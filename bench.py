@@ -15,6 +15,9 @@ Workload (BASELINE.json configs[1], the configuration the metric is quoted on):
              its own roofline, for the record.
 `--impl reference` times the CPU restatement (oracle/, OpenMP over all host threads) of the same
 workload: the reference snapshot has no FFT/FIR block and cannot be built here (DESIGN.md 3).
+`--dump-outputs DIR` writes what the timed path computed in its last step, so that two builds can be
+compared output for output on the same seeded input: DIR/fft4096_window_mag.npy, float32, the
+|FFT| of DUMP_VECTORS of the 32768 vectors (rank 0), picked by a fixed seed.
 
 Multi-GPU: independent per-GPU streams (the path shards by stream / time segment), no
 data-path collective; `scaling` = weak.
@@ -33,6 +36,7 @@ sys.path.insert(0, ROOT)
 N_FFT = 4096
 N_VEC = 32768                       # 32768 x 4096 complex64 = 1 GiB
 SAMPLES = N_FFT * N_VEC
+DUMP_VECTORS = 2048                 # 2048 x 4096 float32 = 32 MiB written by --dump-outputs
 METRIC = "Msamples/s FIR-ccf & FFT-4096 flowgraph at 1/2/4/8 B200; % of HBM/FP32 roofline"
 CONFIG = {
     "workload": "configs[1]: null_source -> fft(N=4096, Blackman-Harris) -> complex_to_mag -> null_sink, "
@@ -297,7 +301,7 @@ def run_reference(args):
     rank, _, world = dist_env()
     if rank != 0:
         return 0
-    steps = max(1, args.steps)
+    steps = args.steps
     cb = cpu_fft_mag_rate(steps, max(0, args.warmup))
     line = {
         "impl": "reference", "metric": METRIC, "value": cb["value"], "unit": "Msamples/s",
@@ -364,7 +368,7 @@ def run_b200(args):
         return float(t.item())
 
     nb.lib()
-    steps, warmup = max(1, args.steps), max(3, args.warmup)
+    steps, warmup = args.steps, max(3, args.warmup)
     peak_gbs, peak_src, peaks = measured_peaks()
     w = blackman_harris(N_FFT)
 
@@ -384,6 +388,13 @@ def run_b200(args):
     ms = timed(torch, lambda: fft.work(x, out), steps, 0, barrier, during=sampler.sample_now)
     sampler.stop()
     launches = nb.launch_count() - l_warm
+    if args.dump_outputs and rank == 0:
+        # before anything else reuses `out`
+        rows = np.sort(np.random.default_rng(0).choice(N_VEC, DUMP_VECTORS, replace=False))
+        sample = out.view(N_VEC, N_FFT)[torch.from_numpy(rows).to(dev)].cpu().numpy()
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "fft4096_window_mag.npy"), sample)
+        del sample
     ms = max_over_ranks(ms)
     value = world * SAMPLES * steps / (ms * 1e-3) / 1e6
     k_ms = ms / steps                                   # one launch per step
@@ -857,7 +868,13 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's output (a seeded sample of its vectors) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the B200 path only")
     claim_stdout()
     if args.impl == "reference":
         return run_reference(args)

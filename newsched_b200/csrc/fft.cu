@@ -19,8 +19,9 @@
 //           table;
 //   pass 3  thread (k1,k0) DFT16 over n0, writes X[k0+16k1+256k2] (coalesced) or |X|.
 // Exactly one HBM read and one HBM write per sample (16 B, or 12 B with the fused |.|).
-// The exchange buffer uses a row stride of 257 complex so all three access patterns are
-// bank-conflict free.
+// fft4096_kernel exchanges through a buffer with a row stride of 257 complex so all three access
+// patterns are bank-conflict free; fft4096_tma_kernel transforms in place in its input tile and
+// swizzles the pass-2 stores instead (see there).
 // Other N (8..8192): generic radix-2 shared-memory Stockham kernel.
 #include <cmath>
 #include <cstdlib>
@@ -32,18 +33,6 @@
 // lifetime of the CTA (measured +5.5 %: 451 -> 476 GS/s fused |.|), 2 = re-fetched before the barrier (-3 %)
 #ifndef B200_FFT_TW2
 #define B200_FFT_TW2 1
-#endif
-// 1 = third barrier moved in front of the pass-1 stores of the next vector (measured -1.5 %)
-// pass-2 -> pass-3 exchange of fft4096_tma_kernel by warp shuffles instead of shared memory (north_star names
-// "warp-shuffle butterflies"): with pass 3 mapped as (k0 = tid >> 4, k1 = tid & 15) the exchange is a 16 x 16
-// transpose inside each group of 16 lanes, four butterfly stages of shfl.xor.  A/B measured on the B200
-// (tools/pk_ab.py, DESIGN.md 4.3): it removes one of the three shared-memory exchanges, and costs 64 SHFL per
-// thread plus stores that are no longer coalesced (lanes then step through k1, i.e. 64 bytes apart).  Default off.
-#ifndef B200_FFT_SHFL
-#define B200_FFT_SHFL 0
-#endif
-#ifndef B200_FFT_LATEBAR
-#define B200_FFT_LATEBAR 0
 #endif
 
 namespace b200 {
@@ -130,25 +119,36 @@ __global__ void __launch_bounds__(256, 2)
     }
 }
 
-// Same three passes, but the NEXT vector is prefetched by the TMA engine (1-D bulk copy, 32 KiB,
-// completion on an mbarrier) into a dedicated shared buffer while passes 2-3 of the current one
-// run: global-load latency is off the critical path and costs no registers or issue slots.
-// smem: sIn 32 KiB | sA 16*257*8 B | sT2 2 KiB | mbarrier  (~67 KiB -> 2-3 CTAs/SM).
-#ifndef B200_FFT_DBUF
-#define B200_FFT_DBUF 0
-#endif
-// Input buffers per CTA.  The fused |.| forms write half as many bytes as they read and are limited
-// on chip: a second buffer (copy issued two vectors ahead) removes the exposed mbarrier wait, +1.8 %
-// (479 -> 487 GS/s).  The complex-output form is HBM-bound and LOSES 11 % with the deeper read
-// prefetch (more reads in flight against the write stream: 408 -> 362 GS/s), so it keeps one.
-#ifndef F4K_NBUF_MAG
-#define F4K_NBUF_MAG 2
-#endif
-constexpr int f4k_nbuf(int out) { return out == B200_FFT_OUT_COMPLEX ? 1 : F4K_NBUF_MAG; }
-constexpr size_t f4k_tma_smem(int out)
-{
-    return (size_t)f4k_nbuf(out) * 4096 * 8 + (B200_FFT_DBUF ? 2 : 1) * 16 * F4K_STRIDE * 8 + 256 * 8 + 32;
-}
+// Same three passes, but the vectors arrive by the TMA engine (1-D bulk copy, 32 KiB, completion on
+// an mbarrier) into NT input tiles, and each vector is transformed IN PLACE in its tile: global-load
+// latency is off the critical path and costs no registers or issue slots, and there is no separate
+// exchange buffer.  Vector i of a CTA (i = 0, 1, ...) uses tile i % NT:
+//   pass 1  thread tid reads tile[n2*256 + tid] and writes its 16 results back to tile[k0*256 + tid]:
+//           the same slots, which no other thread touches, so no barrier between the loads and stores;
+//   -- barrier 1 --
+//   pass 2  row k0 is read and rewritten by the 16 lanes tid >> 4 == k0 alone (half a warp):
+//           __syncwarp() between its loads and its stores; the stores are swizzled (f4k_swz);
+//   -- barrier 2 --
+//   pass 3  thread (k1, k0) reads its 16 contiguous values as 8 LDS.128, conflict-free thanks to the
+//           swizzle.
+// Vector i + 1 lives in another tile, so its pass 1 never touches what pass 3 of vector i reads: no
+// third barrier.  Tile t of vector i is refilled with vector i + NT once every thread has passed
+// barrier 1 of vector i + 1, i.e. once all pass-3 reads of vector i are over; thread 0 is the one
+// that issues that copy, right after the barrier.
+// smem: NT tiles of 32 KiB | sT2 2 KiB | NT mbarriers.
+// Tiles per CTA, i.e. copies in flight = NT - 1 vectors ahead.  The fused |.| forms write half as many
+// bytes as they read and are limited on chip: copies two vectors ahead remove the exposed mbarrier
+// wait (measured +1.8 %, DESIGN.md 4.3).  The complex-output form is HBM-bound and LOSES 11 % with that
+// deeper read prefetch (more reads in flight against the write stream), so its copies stay one vector
+// ahead.
+constexpr int f4k_ntile(int out) { return out == B200_FFT_OUT_COMPLEX ? 2 : 3; }
+constexpr size_t f4k_tma_smem(int out) { return (size_t)f4k_ntile(out) * (4096 * 8 + 8) + 256 * 8; }
+
+// Position of element n0 (0..15) of a 16-element segment of row k0 after the pass-2 stores: the
+// 16-byte chunk index n0 >> 1 is XORed with k0 & 7.  Pass 3 reads a segment as 8 LDS.128 (8 lanes
+// per phase, k0 = 0..7 or 8..15, same k1): unswizzled, all 8 would hit the same chunk of a 2 KiB-
+// aligned row, an 8-way bank conflict; swizzled, they hit 8 different chunks.
+__device__ __forceinline__ int f4k_swz(int n0, int k0) { return (((n0 >> 1) ^ (k0 & 7)) << 1) | (n0 & 1); }
 
 template <bool FWD, int OUT>
 __global__ void __launch_bounds__(256, 2)
@@ -156,21 +156,16 @@ __global__ void __launch_bounds__(256, 2)
                        const float* __restrict__ weff, const float2* __restrict__ tw1,
                        const float2* __restrict__ tw2)
 {
-    constexpr int NBUF = f4k_nbuf(OUT);
+    constexpr int NT = f4k_ntile(OUT);
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    float2* sIn0 = reinterpret_cast<float2*>(smem_raw);
-    float2* sA0 = sIn0 + 4096 * NBUF;
-#if B200_FFT_DBUF
-    float2* sT2 = sA0 + 2 * 16 * F4K_STRIDE;
-#else
-    float2* sT2 = sA0 + 16 * F4K_STRIDE;
-#endif
+    float2* sTile0 = reinterpret_cast<float2*>(smem_raw);
+    float2* sT2 = sTile0 + 4096 * NT;
     uint64_t* bar0 = reinterpret_cast<uint64_t*>(sT2 + 256);
     const int tid = threadIdx.x;
 
     if (tid == 0) {
 #pragma unroll
-        for (int i = 0; i < NBUF; i++)
+        for (int i = 0; i < NT; i++)
             mbar_init(bar0 + i, 1);
         fence_mbar_init();
     }
@@ -196,47 +191,31 @@ __global__ void __launch_bounds__(256, 2)
     pdl_launch_dependents();
     long long vec = blockIdx.x;
     if (tid == 0) {
-        // NBUF input buffers: the copy of vector i + NBUF starts as soon as pass 1 of vector i
-        // has drained its buffer, i.e. more than a whole vector time ahead of its use
+        // the first NT - 1 vectors; the loop then issues one copy per vector, NT - 1 vectors ahead
 #pragma unroll
-        for (int i = 0; i < NBUF; i++)
+        for (int i = 0; i < NT - 1; i++)
             if (vec + (long long)i * gridDim.x < n_vec) {
                 mbar_arrive_expect_tx(bar0 + i, 4096 * 8);
-                bulk_copy_g2s(sIn0 + 4096 * i, in + (vec + (long long)i * gridDim.x) * 4096, 4096 * 8, bar0 + i);
+                bulk_copy_g2s(sTile0 + 4096 * i, in + (vec + (long long)i * gridDim.x) * 4096, 4096 * 8, bar0 + i);
             }
     }
-    uint32_t phase = 0;
-    int it = 0;
-    for (; vec < n_vec; vec += gridDim.x, it++) {
+    int t = 0;        // tile of this CTA's vector i: i % NT
+    uint32_t par = 0; // parity of that tile's mbarrier phase: (i / NT) & 1
+    for (; vec < n_vec; vec += gridDim.x) {
         float2 v[16];
-        float2* sIn = sIn0 + (NBUF == 2 ? (it & 1) * 4096 : 0);
-        uint64_t* bar = bar0 + (NBUF == 2 ? (it & 1) : 0);
-        const uint32_t par = NBUF == 2 ? (uint32_t)((it >> 1) & 1) : phase;
-#if B200_FFT_DBUF
-        // two exchange buffers, alternating per vector: the pass-1 stores of this vector cannot hit
-        // rows another warp is still reading for the previous one, so the third barrier goes away
-        float2* sA = sA0 + (phase ? 16 * F4K_STRIDE : 0);
-#else
-        float2* sA = sA0;
-#endif
-        mbar_wait(bar, par);
-        phase ^= 1;
+        float2* tile = sTile0 + t * 4096;
+        mbar_wait(bar0 + t, par);
+        // ---- pass 1: over n2, thread = L = n1*16+n0, results back into the slots it read
 #pragma unroll
         for (int i = 0; i < 16; i++)
-            v[i] = sIn[i * 256 + tid];
+            v[i] = tile[i * 256 + tid];
 #pragma unroll
         for (int i = 0; i < 16; i++)
             v[i] = __fmul2_rn(v[i], make_float2(wreg[i], wreg[i]));
         dft16<FWD>(v);
-#if B200_FFT_LATEBAR
-        // pass-3 reads of the previous vector must be over before sA is overwritten: waiting HERE
-        // instead of at the end of the loop lets the loads, the window and the first DFT16 of this
-        // vector run while slower warps are still storing the previous one
-        __syncthreads();
-#endif
 #pragma unroll
         for (int k0 = 0; k0 < 16; k0++)
-            sA[k0 * F4K_STRIDE + tid] = cmul(v[pos16(k0)], t1[k0]);
+            tile[k0 * 256 + tid] = cmul(v[pos16(k0)], t1[k0]);
 #if B200_FFT_TW2 == 2
         // v[] is dead until pass 2 reloads it: fetch this thread's pass-2 twiddles now, so that the
         // barrier below covers their shared-memory latency
@@ -245,86 +224,44 @@ __global__ void __launch_bounds__(256, 2)
         for (int k1 = 1; k1 < 16; k1++)
             t2r[k1] = sT2[k1 * 16 + (tid & 15)];
 #endif
-        __syncthreads(); // sA complete; every thread is done reading sIn
-        if (tid == 0 && vec + (long long)NBUF * gridDim.x < n_vec) {
-            mbar_arrive_expect_tx(bar, 4096 * 8);
-            bulk_copy_g2s(sIn, in + (vec + (long long)NBUF * gridDim.x) * 4096, 4096 * 8, bar);
+        __syncthreads(); // rows complete for pass 2; every thread is past pass 3 of the previous vector
+        const int tn = t == 0 ? NT - 1 : t - 1; // the previous vector's tile, now free
+        if (tid == 0 && vec + (long long)(NT - 1) * gridDim.x < n_vec) {
+            fence_proxy_async(); // the generic-proxy accesses of that tile before the async-proxy copy into it
+            mbar_arrive_expect_tx(bar0 + tn, 4096 * 8);
+            bulk_copy_g2s(sTile0 + tn * 4096, in + (vec + (long long)(NT - 1) * gridDim.x) * 4096, 4096 * 8,
+                          bar0 + tn);
         }
-#if B200_FFT_SHFL
+        // ---- pass 2: over n1, thread = (k0, n0), in place within row k0
         {
             const int k0 = tid >> 4, n0 = tid & 15;
-            const float2* row = sA + k0 * F4K_STRIDE + n0;
+            float2* row = tile + k0 * 256;
 #pragma unroll
             for (int i = 0; i < 16; i++)
-                v[i] = row[i * 16];
+                v[i] = row[i * 16 + n0];
+            __syncwarp(); // the other 15 lanes of this row have read it before it is overwritten
             dft16<FWD>(v);
-            float2 w[16];
-            w[0] = v[pos16(0)];
-#pragma unroll
-            for (int k1 = 1; k1 < 16; k1++)
-                w[k1] = cmul(v[pos16(k1)], t2r[k1]);
-            // 16 x 16 transpose inside the 16-lane group: afterwards w[i] = the value lane i held for k1 = my lane
-#pragma unroll
-            for (int sft = 1; sft < 16; sft <<= 1) {
-                const bool up = (n0 & sft) != 0;
-#pragma unroll
-                for (int i = 0; i < 16; i++) {
-                    if (i & sft)
-                        continue;
-                    const float2 send = up ? w[i] : w[i | sft];
-                    float2 recv;
-                    recv.x = __shfl_xor_sync(0xffffffffu, send.x, sft);
-                    recv.y = __shfl_xor_sync(0xffffffffu, send.y, sft);
-                    if (up)
-                        w[i] = recv;
-                    else
-                        w[i | sft] = recv;
-                }
-            }
-#pragma unroll
-            for (int i = 0; i < 16; i++)
-                v[i] = w[i];
-            dft16<FWD>(v);
-            const int k1 = n0; // this thread now owns (k0, k1): X[k0 + 16 k1 + 256 k2]
-            if (OUT == B200_FFT_OUT_COMPLEX) {
-                float2* y = reinterpret_cast<float2*>(out) + vec * 4096;
-#pragma unroll
-                for (int k2 = 0; k2 < 16; k2++)
-                    __stcs(y + k2 * 256 + k1 * 16 + k0, v[pos16(k2)]);
-            } else {
-                float* y = reinterpret_cast<float*>(out) + vec * 4096;
-#pragma unroll
-                for (int k2 = 0; k2 < 16; k2++) {
-                    float2 z = v[pos16(k2)];
-                    float p = fmaf(z.x, z.x, z.y * z.y);
-                    __stcs(y + k2 * 256 + k1 * 16 + k0, OUT == B200_FFT_OUT_MAG ? sqrt_approx(p) : p);
-                }
-            }
-        }
-#else
-        {
-            const int k0 = tid >> 4, n0 = tid & 15;
-            float2* row = sA + k0 * F4K_STRIDE + n0;
-#pragma unroll
-            for (int i = 0; i < 16; i++)
-                v[i] = row[i * 16];
-            dft16<FWD>(v);
-            row[0] = v[pos16(0)];
+            float2* dst = row + f4k_swz(n0, k0);
+            dst[0] = v[pos16(0)];
 #pragma unroll
             for (int k1 = 1; k1 < 16; k1++)
 #if B200_FFT_TW2
-                row[k1 * 16] = cmul(v[pos16(k1)], t2r[k1]);
+                dst[k1 * 16] = cmul(v[pos16(k1)], t2r[k1]);
 #else
-                row[k1 * 16] = cmul(v[pos16(k1)], sT2[k1 * 16 + n0]);
+                dst[k1 * 16] = cmul(v[pos16(k1)], sT2[k1 * 16 + n0]);
 #endif
         }
         __syncthreads();
+        // ---- pass 3: over n0, thread = (k1, k0)
         {
-            const int k0 = tid & 15, k1 = tid >> 4;
-            const float2* row = sA + k0 * F4K_STRIDE + k1 * 16;
+            const int k0 = tid & 15, k1 = tid >> 4, s = k0 & 7;
+            const float4* seg = reinterpret_cast<const float4*>(tile + k0 * 256 + k1 * 16);
 #pragma unroll
-            for (int i = 0; i < 16; i++)
-                v[i] = row[i];
+            for (int j = 0; j < 8; j++) {
+                const float4 q = seg[j ^ s];
+                v[2 * j] = make_float2(q.x, q.y);
+                v[2 * j + 1] = make_float2(q.z, q.w);
+            }
             dft16<FWD>(v);
             if (OUT == B200_FFT_OUT_COMPLEX) {
                 float2* y = reinterpret_cast<float2*>(out) + vec * 4096;
@@ -341,10 +278,10 @@ __global__ void __launch_bounds__(256, 2)
                 }
             }
         }
-#endif
-#if !B200_FFT_LATEBAR && !B200_FFT_DBUF
-        __syncthreads();
-#endif
+        if (++t == NT) {
+            t = 0;
+            par ^= 1;
+        }
     }
 }
 

@@ -1075,6 +1075,13 @@ using namespace b200;
 #define PFB64_TC_DEFAULT 0
 #endif
 
+// MaxDynamicSharedMemorySize of every channelizer kernel: the most a block may have on sm_100.  The attribute belongs
+// to the kernel, and handles with different shared-memory sizes share an instantiation (pfb64_kernel<0> at P = 20
+// and 28, every pfb_generic_kernel handle, ...): a per-handle value set by the last b200_pfb_create would make the
+// launches of an older, larger handle fail.  Each launch passes its own h->smem, which the create-time checks keep
+// within 220 KiB (227 KiB for the two-tile pfbm_kernel).
+constexpr int PFB_SMEM_ATTR = 227 * 1024;
+
 // shared memory of pfbs_kernel: one (padded) input tile, and everything else
 static inline size_t pfbs_xbytes(int M, int P4)
 {
@@ -1307,13 +1314,13 @@ int b200_pfb_create(const b200_pfb_params* p, b200_pfb** out)
             b200_pfb_destroy(h);
             return set_err(B200_ERR_UNSUPPORTED, "pfb_create: taps_per_channel too large for M=64 tile");
         }
-        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<24>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
+        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
+        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
+        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
+        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
+        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<24>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
+        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
         h->grid = 2 * sm_count();
         if (h->P4 <= 16) {
             // tensor-core DFT form: DFT matrix rows m = 2c + part; columns k = 2i + (re | im) for the K-major planes,
@@ -1335,10 +1342,10 @@ int b200_pfb_create(const b200_pfb_params* p, b200_pfb** out)
             PFB_CUDA(cudaMalloc(&h->d_dft, F.size() * 2));
             PFB_CUDA(cudaMemcpy(h->d_dft, F.data(), F.size() * 2, cudaMemcpyHostToDevice));
             h->smem_tc = 1024 + 2 * (size_t)PFBT_PLANE + 2 * sizeof(float2) * (size_t)rows * 64 + 64;
-            PFB_CUDA(cudaFuncSetAttribute(pfb64_tc_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_tc));
-            PFB_CUDA(cudaFuncSetAttribute(pfb64_tc_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_tc));
-            PFB_CUDA(cudaFuncSetAttribute(pfb64_tc_kernel<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_tc));
-            PFB_CUDA(cudaFuncSetAttribute(pfb64_tc_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_tc));
+            PFB_CUDA(cudaFuncSetAttribute(pfb64_tc_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
+            PFB_CUDA(cudaFuncSetAttribute(pfb64_tc_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
+            PFB_CUDA(cudaFuncSetAttribute(pfb64_tc_kernel<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
+            PFB_CUDA(cudaFuncSetAttribute(pfb64_tc_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
             h->tc_ok = 1;
             h->tc = PFB64_TC_DEFAULT;
             if (const char* e = getenv("B200_PFB_TC"))
@@ -1350,10 +1357,10 @@ int b200_pfb_create(const b200_pfb_params* p, b200_pfb** out)
         h->nbuf = (2 * pfbs_xbytes(M, h->P4) + pfbs_rest(M, h->P4) <= 113 * 1024 && !getenv("B200_PFB_ONEBUF")) ? 2 : 1;
         h->smem = h->nbuf * pfbs_xbytes(M, h->P4) + pfbs_rest(M, h->P4);
 #define PFBS_ATTR(MM)                                                                                          \
-    PFB_CUDA(cudaFuncSetAttribute(pfbs_kernel<MM, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem)); \
-    PFB_CUDA(cudaFuncSetAttribute(pfbs_kernel<MM, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem)); \
-    PFB_CUDA(cudaFuncSetAttribute(pfbs_kernel<MM, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem)); \
-    PFB_CUDA(cudaFuncSetAttribute(pfbs_kernel<MM, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem))
+    PFB_CUDA(cudaFuncSetAttribute(pfbs_kernel<MM, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR)); \
+    PFB_CUDA(cudaFuncSetAttribute(pfbs_kernel<MM, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR)); \
+    PFB_CUDA(cudaFuncSetAttribute(pfbs_kernel<MM, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR)); \
+    PFB_CUDA(cudaFuncSetAttribute(pfbs_kernel<MM, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR))
         if (M == 8) {
             PFBS_ATTR(8);
         } else {
@@ -1373,10 +1380,10 @@ int b200_pfb_create(const b200_pfb_params* p, b200_pfb** out)
         h->nbuf = (M >= 128 && 2 * xbytes + rest <= 227 * 1024 && !getenv("B200_PFB_ONEBUF")) ? 2 : 1;
         h->smem = h->nbuf * xbytes + rest;
 #define PFBM_ATTR(MM)                                                                                          \
-    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem)); \
-    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem)); \
-    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem)); \
-    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem))
+    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR)); \
+    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR)); \
+    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR)); \
+    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR))
         if (M == 16) {
             PFBM_ATTR(16);
         } else if (M == 32) {
@@ -1398,8 +1405,7 @@ int b200_pfb_create(const b200_pfb_params* p, b200_pfb** out)
             b200_pfb_destroy(h);
             return set_err(B200_ERR_UNSUPPORTED, "pfb_create: taps_per_channel too large");
         }
-        PFB_CUDA(cudaFuncSetAttribute(pfb_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)h->smem));
+        PFB_CUDA(cudaFuncSetAttribute(pfb_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
         if (M >= 16) {
             b200_fft_params fp{};
             fp.n = M;

@@ -156,8 +156,7 @@ typedef struct {
     int32_t fuse_multiply_const; /* 0/1 */
     float k_re, k_im;     /* epilogue constant (k_im ignored for fff) */
     int32_t algorithm;    /* 0 = auto, 1 = direct SIMT, 2 = block-Toeplitz GEMM on the tensor cores (tcgen05; ccf with D <= 8, fff with D = 1 and <= 449 taps), 3 = overlap-save FFT,
-                             4 = one thread per output (fallback), 5 = 2-parallel fast FIR (decimation 1),
-                             6 = algorithm 2 with TF32 operands (measurement variant: ~1e-7 rel. RMS, several times slower) */
+                             4 = one thread per output (fallback); any other value is rejected with B200_ERR_ARG */
 } b200_fir_params;
 B200_API int b200_fir_create(const b200_fir_params* p, b200_fir** h);
 B200_API int b200_fir_destroy(b200_fir* h);

@@ -86,9 +86,7 @@ struct b200_fir {
     int dg = 0;      // > 1: decimation by a non-divisor of 16 folded into the full-rate kernel (D rows per thread)
     int dd = 0;      // > 1: decimation folded into the TMA-staged full-rate kernel (geometry as for D = 1)
     ols_plan* ols = nullptr; // algorithm 3
-    tc_plan* tc = nullptr;   // algorithm 2 (bf16 split) / 6 (tf32 split)
-    int tc_tf32 = 0;
-    ffa_plan* ffa = nullptr; // algorithm 5
+    tc_plan* tc = nullptr;   // algorithm 2
     int algorithm = 1;
     fir_epilogue ep{ 0, 1.f, 0.f };
     float* d_taps_pp = nullptr; // [D][TQ] reversed per phase
@@ -127,8 +125,6 @@ static int fir_launch(b200_fir* h, const float* d_hist, const void* d_in, void* 
         return ols_launch(h->ols, d_hist, d_in, d_out, n_in, n_out, s);
     if (h->algorithm == 2)
         return tc_launch(h->tc, d_hist, d_in, d_out, n_in, n_out, s);
-    if (h->algorithm == 5)
-        return ffa_launch(h->ffa, d_hist, d_in, d_out, n_in, n_out, s);
     if (h->algorithm == 1 && h->rp) {
         // real stream as float pairs: tiles of 2048 pairs = 4096 real outputs
         const long long pairs_out = (n_out + 1) / 2, pairs_in = (n_in + 1) / 2;
@@ -431,7 +427,6 @@ int b200_fir_destroy(b200_fir* h)
     cudaFree(h->d_hist[1]);
     ols_destroy(h->ols);
     tc_destroy(h->tc);
-    ffa_destroy(h->ffa);
     delete h;
     return B200_OK;
 }
@@ -443,6 +438,9 @@ int b200_fir_create(const b200_fir_params* p, b200_fir** out)
     *out = nullptr;
     if (!p->taps || p->n_taps < 1 || p->decimation < 1)
         return set_err(B200_ERR_ARG, "fir_create: need n_taps >= 1, decimation >= 1, taps != NULL");
+    if (p->algorithm < 0 || p->algorithm > 4)
+        return set_err(B200_ERR_ARG, "fir_create: algorithm must be 0 (auto), 1 (direct SIMT), 2 (tensor core), 3 (overlap-save) "
+                                     "or 4 (one thread per output)");
     if (p->algorithm == 2 && !tc_supported(p->n_taps, p->decimation, !p->is_complex))
         return set_err(B200_ERR_UNSUPPORTED,
                        "fir_create: the tensor-core form needs decimation 1..8 and <= 2048 taps per branch (complex stream), or "
@@ -499,36 +497,10 @@ int b200_fir_create(const b200_fir_params* p, b200_fir** out)
         bool want2 = p->algorithm == 2;
         if (p->algorithm == 0 && h->vec == 2 && h->D == 1 && h->T >= 33 && h->T <= 384 && tc_supported(h->T, h->D, 0))
             want2 = true;
-        // float streams (fff): the same kernel with two 4096-sample runs per tile; crossovers measured with
-        // tools/real_tc_ab.py (B200_FIR_REAL_TC_MIN / _MAX override them)
-        if (p->algorithm == 0 && h->vec == 1 && h->D == 1 && tc_supported(h->T, h->D, 1)) {
-            int tmin = 33, tmax = 448;
-            if (const char* e = getenv("B200_FIR_REAL_TC_MIN"))
-                tmin = atoi(e);
-            if (const char* e = getenv("B200_FIR_REAL_TC_MAX"))
-                tmax = atoi(e);
-            if (h->T >= tmin && h->T <= tmax)
-                want2 = true;
-        }
-        if (const char* e = getenv("B200_FIR_ALGO")) {
-            if (p->algorithm == 0 && atoi(e) == 2 && tc_supported(h->T, h->D, h->vec == 1))
-                want2 = true;
-            else if (p->algorithm == 0 && atoi(e) != 0)
-                want2 = false;
-        }
-        if (p->algorithm == 6) { // TF32 measurement variant of the same formulation
-            if (h->vec != 2 || h->D != 1) {
-                b200_fir_destroy(h);
-                return set_err(B200_ERR_UNSUPPORTED, "fir_create: the tf32 tensor-core variant needs a complex stream and decimation 1");
-            }
-            int rc = tc_create_tf32(p->taps, h->T, h->ep.fuse, h->ep.kre, h->ep.kim, &h->tc);
-            if (rc != B200_OK) {
-                b200_fir_destroy(h);
-                return rc;
-            }
-            h->algorithm = 2;
-            h->tc_tf32 = 1;
-        } else if (want2) {
+        // float streams (fff): the same kernel with two 4096-sample runs per tile; crossovers measured with tools/real_tc_ab.py
+        if (p->algorithm == 0 && h->vec == 1 && h->D == 1 && h->T >= 33 && h->T <= 448 && tc_supported(h->T, h->D, 1))
+            want2 = true;
+        if (want2) {
             int rc = tc_create(p->taps, h->T, h->D, h->vec == 1, h->ep.fuse, h->ep.kre, h->ep.kim, &h->tc);
             if (rc != B200_OK) {
                 b200_fir_destroy(h);
@@ -585,9 +557,6 @@ int b200_fir_create(const b200_fir_params* p, b200_fir** out)
                 tx = h->dd == 2 ? 256 : h->dd == 4 ? 512 : 768;
             want = can && h->T > tx;
         }
-        if (const char* e = getenv("B200_FIR_ALGO"))
-            if (p->algorithm == 0)
-                want = atoi(e) == 3;
         if (h->algorithm == 2)
             want = false; // the tensor-core form was chosen above
         if (want && !can && p->algorithm == 3) {
@@ -602,34 +571,6 @@ int b200_fir_create(const b200_fir_params* p, b200_fir** out)
             }
             h->algorithm = 3;
         }
-    }
-
-    // 2-parallel fast FIR (algorithm 5): full-rate filters in the FP32-bound range below the
-    // overlap-save crossover execute 0.77x the FMAs of the direct form
-    if (h->algorithm == 1 && h->D == 1) {
-        const bool can5 = ffa_supported(h->T, h->D, h->vec == 1);
-        bool want5 = p->algorithm == 5;
-        // measured (tools/ffa_sweep.py): 0.70x the per-tap cost of the direct form but 3x its fixed
-        // cost per tile, so it loses below ~100 taps (64 taps: 192 vs 214 GS/s) and overlap-save wins
-        // above: never picked automatically, kept selectable (algorithm = 5 / B200_FIR_ALGO=5)
-        if (const char* e = getenv("B200_FIR_ALGO"))
-            if (p->algorithm == 0)
-                want5 = atoi(e) == 5;
-        if (p->algorithm == 5 && !can5) {
-            b200_fir_destroy(h);
-            return set_err(B200_ERR_UNSUPPORTED, "fir_create: the 2-parallel form needs decimation 1 and 4..2048 taps");
-        }
-        if (want5 && can5) {
-            int rc = ffa_create(p->taps, h->T, h->vec == 1, h->ep.fuse, h->ep.kre, h->ep.kim, &h->ffa);
-            if (rc != B200_OK) {
-                b200_fir_destroy(h);
-                return rc;
-            }
-            h->algorithm = 5;
-        }
-    } else if (p->algorithm == 5) {
-        b200_fir_destroy(h);
-        return set_err(B200_ERR_UNSUPPORTED, "fir_create: the 2-parallel form needs decimation 1");
     }
 
 #define FIR_CUDA(call)                                                                   \
@@ -704,7 +645,7 @@ int b200_fir_create(const b200_fir_params* p, b200_fir** out)
     return B200_OK;
 }
 
-int b200_fir_algorithm(const b200_fir* h) { return h ? (h->tc_tf32 ? 6 : h->algorithm) : 0; }
+int b200_fir_algorithm(const b200_fir* h) { return h ? h->algorithm : 0; }
 
 int b200_fir_geometry(const b200_fir* h, int* decimation, int* item_bytes)
 {

@@ -10,7 +10,6 @@
 #include <vector>
 
 #include "common.cuh"
-#include "fir_ffa.cuh"
 #include "fir_interp.cuh"
 #include "fir_ols.cuh"
 #include "fir_tc.cuh"

@@ -6,8 +6,8 @@
 // block interface this stands behind is gr::block::work, runtime/include/gnuradio/block.hpp:81-85.
 // BASELINE.json north_star: "long-tap FIR expressed as Toeplitz/polyphase GEMM".
 //
-// Formulation.  Real taps act on the real and the imaginary stream separately, so a tile of 8192
-// outputs is two real problems (planes "re" and "im").  Write an output index as m = 64 r + c
+// Formulation.  Real taps act on the real and the imaginary stream separately, so a tile of outputs
+// is two real problems (planes "re" and "im").  Write an output index in the tile as m = 64 r + c
 // (r = 0..127, c = 0..63) and, per polyphase branch p (h_p[q] = h[qD+p], x_p[j] = x[jD-p]),
 //
 //     Y[c][r] = sum_j  A_p[c][j] * X_p[r][j],   A_p[c][j] = h_p[c + P - j],   X_p[r][j] = xs_p[64 r + j]
@@ -18,21 +18,27 @@
 // ONCE, linearly (in that swizzle), and the 128 x K operand the MMA reads is produced by the shared
 // memory descriptor alone: K-atom a / K-step t start at byte a*128 + t*32 of the plane.  No im2col
 // copy exists anywhere.  A_p (64 phases x K, a Toeplitz band of the taps) is built on the host at
-// create time, pre-swizzled, and streamed from L2 by 1-D bulk copies (16 KiB per 64-wide K-atom).
+// create time.
 //
 // Precision.  fp32 -> bf16 hi + bf16 lo (x = hi + lo + O(2^-18 |x|)).  The tap operand carries
 // [h_hi phases 0..63 ; h_lo phases 0..63] as its M = 128 rows, the signal operand is x_hi, then x_lo:
-// two 128x128x16 MMAs per K-step per plane give all FOUR partial products (hi*hi, hi*lo, lo*hi, lo*lo) in
-// TMEM lanes c and 64+c, which the epilogue adds.  fp32 accumulation in TMEM.
+// two MMAs per K-step per plane give all FOUR partial products (hi*hi, hi*lo, lo*hi, lo*lo), and the
+// epilogue adds the hi-tap and the lo-tap sums of each phase.  fp32 accumulation in TMEM.
 //
-// One CTA = one tile of 8192 outputs; 128 threads: all convert (fp32 -> 4 swizzled bf16 planes in
-// shared memory), warp 0 issues the MMAs, warp 1 streams the tap atoms, all four warps drain TMEM
-// (warp w owns lanes 32w..32w+31), combine the hi-/lo-tap halves through shared memory and leave
-// by one bulk store.  256 TMEM columns and ~100 KB of shared memory per CTA -> two CTAs per SM, so
-// one CTA's conversion / epilogue overlaps the other's MMAs.
+// Two kernels run this formulation.  Both are persistent (one CTA per SM) and warp-specialised, so the
+// conversion (fp32 -> 4 swizzled bf16 planes in shared memory), the MMAs and the epilogue of successive
+// tiles overlap; each is described above its code.
+//   fir_tc_ts_kernel    tap-stationary: decimation 1 and K <= 512 (up to 449 taps).  The taps sit in tensor
+//                       memory for the whole call and tiles are 4096 outputs.  A float stream, which only
+//                       this kernel takes, runs 8192 per tile: two 4096-sample runs ride through the planes
+//                       "re" and "im", the same MMAs at twice the sample rate.  tc_create picks this kernel
+//                       whenever it applies, so auto selection (at most 448 taps) reaches only this one.
+//   fir_tc_pipe_kernel  ring form: decimation 1..8, up to 2048 taps per branch, tiles of 8192 outputs.  The
+//                       pre-swizzled tap atoms stream from L2 through a shared-memory ring by 1-D bulk
+//                       copies (16 KiB per 64-wide K-atom).  It serves explicit algorithm 2 at D > 1 or
+//                       beyond 449 taps.
 #include <cuda_bf16.h>
 
-#include <algorithm>
 #include <vector>
 
 #include "common.cuh"
@@ -45,10 +51,12 @@ constexpr int TC_NROW = 128;             // signal rows per tile (MMA N)
 constexpr int TC_PH = 64;                // outputs per row = bf16 elements per 128-byte swizzle row
 constexpr int TC_TILE = TC_NROW * TC_PH; // outputs per tile
 constexpr int TC_ATOM_BYTES = 128 * 128; // one K-atom of the tap operand: 128 rows x 64 bf16
-constexpr int TC_THREADS = 128;
 constexpr int TC_TMEM_COLS = 256;        // re accumulator: columns 0..127, im: 128..255
 constexpr int TC_MAX_STAGES = 4;
 
+// Both kernels take this as a __grid_constant__ and read it in place from the parameter bank.  As a plain by-value
+// struct, how the compiler stages it depends on its size: at this size the float-stream converter loop came out
+// 4 instructions longer and fir_fff at 64 taps ran 1.2 % slower (B200, 1000 W power limit).
 struct tc_args {
     const float2* x;
     const float2* hist;
@@ -65,386 +73,12 @@ struct tc_args {
     int stages;      // tap-atom ring depth
     int fuse;
     float kre, kim;
-    int desc_mode;   // 0: base_offset field 0 (swizzle on absolute address bits); 1: base_offset = (addr >> 7) & 7
     const uint32_t* gAt; // TMEM-resident form: tap matrix [128 lanes][16*ksteps / 2] bf16 pairs, K contiguous
     int ts_plane_elems, ts_plane_bytes, ts_stages, ts_stage_bytes;
-    int ts_swap;     // diagnostic: swap the bf16 halves of every 32-bit TMEM column of A
-    int real;        // fff (float stream): a tile is 8192 real outputs = two 4096-sample runs riding through the two planes
-                     // ("re" = first run, "im" = second) of the complex kernel: same MMAs, twice the sample rate
-    int ts_nohead;   // A/B: head tile through the element-wise path (B200_TC_TS_HEAD=0)
-    int ts_pdl;      // launched with programmatic stream serialization: griddepcontrol.wait after the prologue
-    int dbg;         // bottleneck attribution (B200_TC_DBG): 1 = skip conversion, 2 = skip epilogue, 4 = skip MMAs, 8 = skip input copies
 };
 
 // instruction descriptor: bf16 x bf16 -> fp32, both operands K-major, M = 128, N = 128
 constexpr uint32_t TC_IDESC = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(TC_NROW >> 3) << 17) | ((128u >> 4) << 24);
-
-
-__global__ void __launch_bounds__(TC_THREADS, 2) fir_tc_kernel(const tc_args a)
-{
-    extern __shared__ uint8_t tc_smem_raw[];
-    uint8_t* smem = tc_align1024(tc_smem_raw);
-    uint8_t* planes = smem;                                   // [re_hi][re_lo][im_hi][im_lo]
-    uint8_t* ring = smem + 4 * (size_t)a.plane_bytes;         // tap atoms
-    uint64_t* bars = reinterpret_cast<uint64_t*>(ring + (size_t)a.stages * TC_ATOM_BYTES);
-    uint64_t* full = bars;                                    // [stages]
-    uint64_t* empty = bars + TC_MAX_STAGES;                   // [stages]
-    uint64_t* round_done = bars + 2 * TC_MAX_STAGES;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * TC_MAX_STAGES + 1);
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const long long m0 = (long long)blockIdx.x * TC_TILE;
-    const int total_atoms = a.D * a.KA;
-
-    if (tid == 0) {
-        for (int s = 0; s < a.stages; s++) {
-            mbar_init(&full[s], 1);
-            mbar_init(&empty[s], 1);
-        }
-        mbar_init(round_done, 1);
-        fence_mbar_init();
-    }
-    if (warp == 0) {
-        __syncwarp();
-        tc_alloc(tmem_slot, TC_TMEM_COLS);
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = *tmem_slot;
-
-    // warp 1 starts streaming the tap atoms right away (they do not depend on the conversion)
-    int prod_next = 0;
-    if (warp == 1) {
-        for (; prod_next < total_atoms && prod_next < a.stages; prod_next++) {
-            if (lane == 0) {
-                mbar_arrive_expect_tx(&full[prod_next], TC_ATOM_BYTES);
-                bulk_copy_g2s(ring + (size_t)prod_next * TC_ATOM_BYTES, a.gA + (size_t)prod_next * TC_ATOM_BYTES,
-                              TC_ATOM_BYTES, &full[prod_next]);
-            }
-        }
-        __syncwarp();
-    }
-
-    const uint32_t planes_s = smem_u32(planes);
-    const uint32_t ring_s = smem_u32(ring);
-
-    for (int p = 0; p < a.D; p++) {
-        if (p > 0) { // the previous branch's MMAs must have finished reading the planes
-            mbar_wait(round_done, (p - 1) & 1);
-            tc_fence_after();
-        }
-        // ---- conversion: branch samples xs[i] = x[(m0 - P + i) * D - p] -> bf16 hi / lo planes
-        {
-            const long long j0 = m0 - a.P;
-            const bool fast = a.D == 1 && j0 >= 0 && j0 + a.plane_elems <= a.n_in &&
-                              (reinterpret_cast<uintptr_t>(a.x) & 15) == 0;
-            if (fast) {
-                const float4* src = reinterpret_cast<const float4*>(a.x + j0);
-                const int npairs = a.plane_elems >> 1;
-#pragma unroll 1
-                for (int base = 0; base < npairs; base += TC_THREADS * 8) {
-                    float4 v[8];
-#pragma unroll
-                    for (int u = 0; u < 8; u++) {
-                        const int q = base + u * TC_THREADS + tid;
-                        v[u] = q < npairs ? __ldg(src + q) : make_float4(0.f, 0.f, 0.f, 0.f);
-                    }
-#pragma unroll
-                    for (int u = 0; u < 8; u++) {
-                        const int q = base + u * TC_THREADS + tid;
-                        if (q < npairs) {
-                            const __nv_bfloat162 rh = __floats2bfloat162_rn(v[u].x, v[u].z);
-                            const __nv_bfloat162 ih = __floats2bfloat162_rn(v[u].y, v[u].w);
-                            const float2 rhf = __bfloat1622float2(rh), ihf = __bfloat1622float2(ih);
-                            const __nv_bfloat162 rl = __floats2bfloat162_rn(v[u].x - rhf.x, v[u].z - rhf.y);
-                            const __nv_bfloat162 il = __floats2bfloat162_rn(v[u].y - ihf.x, v[u].w - ihf.y);
-                            const uint32_t off = tc_plane_off(2u * q);
-                            *reinterpret_cast<__nv_bfloat162*>(planes + off) = rh;
-                            *reinterpret_cast<__nv_bfloat162*>(planes + a.plane_bytes + off) = rl;
-                            *reinterpret_cast<__nv_bfloat162*>(planes + 2 * a.plane_bytes + off) = ih;
-                            *reinterpret_cast<__nv_bfloat162*>(planes + 3 * a.plane_bytes + off) = il;
-                        }
-                    }
-                }
-            } else {
-#pragma unroll 4
-                for (int i = tid; i < a.plane_elems; i += TC_THREADS) {
-                    const long long n = (j0 + i) * a.D - p;
-                    float2 v = make_float2(0.f, 0.f);
-                    if (n >= 0) {
-                        if (n < a.n_in)
-                            v = __ldg(a.x + n);
-                    } else if (a.hist != nullptr && n >= -(long long)a.Tm1) {
-                        v = __ldg(a.hist + (a.Tm1 + n));
-                    }
-                    __nv_bfloat16 rh, rl, ih, il;
-                    tc_split(v.x, rh, rl);
-                    tc_split(v.y, ih, il);
-                    const uint32_t off = tc_plane_off((uint32_t)i);
-                    *reinterpret_cast<__nv_bfloat16*>(planes + off) = rh;
-                    *reinterpret_cast<__nv_bfloat16*>(planes + a.plane_bytes + off) = rl;
-                    *reinterpret_cast<__nv_bfloat16*>(planes + 2 * a.plane_bytes + off) = ih;
-                    *reinterpret_cast<__nv_bfloat16*>(planes + 3 * a.plane_bytes + off) = il;
-                }
-            }
-        }
-        fence_proxy_async(); // generic-proxy stores -> visible to the tensor core's async-proxy reads
-        __syncthreads();
-
-        if (warp == 0) {
-            // ---- MMA issue: per K-step, (re, im) x (x_hi, x_lo) against the [h_hi ; h_lo] tap rows
-            for (int at = 0; at < a.KA; at++) {
-                const int g = p * a.KA + at, s = g % a.stages, use = g / a.stages;
-                mbar_wait(&full[s], use & 1);
-                tc_fence_after();
-                if (lane == 0) {
-                    const int nst = min(4, a.ksteps - 4 * at);
-                    for (int t = 0; t < nst; t++) {
-                        const uint64_t adesc = tc_desc(ring_s + s * TC_ATOM_BYTES + t * 32, a.desc_mode);
-                        const uint32_t boff = at * 128 + t * 32;
-                        const uint32_t acc = (g | t) != 0;
-                        tc_mma_bf16(tmem, adesc, tc_desc(planes_s + boff, a.desc_mode), TC_IDESC, acc);
-                        tc_mma_bf16(tmem, adesc, tc_desc(planes_s + a.plane_bytes + boff, a.desc_mode), TC_IDESC, 1);
-                        tc_mma_bf16(tmem + TC_NROW, adesc, tc_desc(planes_s + 2 * a.plane_bytes + boff, a.desc_mode),
-                                    TC_IDESC, acc);
-                        tc_mma_bf16(tmem + TC_NROW, adesc, tc_desc(planes_s + 3 * a.plane_bytes + boff, a.desc_mode),
-                                    TC_IDESC, 1);
-                    }
-                    tc_commit(&empty[s]); // the atom's slot is free once these MMAs have read it
-                    if (at == a.KA - 1)
-                        tc_commit(round_done);
-                }
-                __syncwarp();
-            }
-        } else if (warp == 1) {
-            // ---- tap-atom producer: refill slots as the MMAs release them (runs ahead across branches)
-            const int upto = min(total_atoms, (p + 1) * a.KA + a.stages);
-            for (; prod_next < upto; prod_next++) {
-                const int s = prod_next % a.stages, use = prod_next / a.stages;
-                mbar_wait(&empty[s], (use & 1) ^ 1);
-                if (lane == 0) {
-                    mbar_arrive_expect_tx(&full[s], TC_ATOM_BYTES);
-                    bulk_copy_g2s(ring + (size_t)s * TC_ATOM_BYTES, a.gA + (size_t)prod_next * TC_ATOM_BYTES,
-                                  TC_ATOM_BYTES, &full[s]);
-                }
-                __syncwarp();
-            }
-        }
-    }
-    mbar_wait(round_done, (a.D - 1) & 1);
-    tc_fence_after();
-
-    // ---- epilogue: TMEM lane 32w + l = tap-part (w >> 1), phase c; column r -> output 64 r + c.
-    // The output tile (8192 complex64 = 64 KiB) reuses the plane storage.
-    float2* tile = reinterpret_cast<float2*>(planes);
-    const int c = tid & 63, part = warp >> 1;
-    const uint32_t tl = tmem + ((uint32_t)(warp * 32) << 16);
-#pragma unroll 1
-    for (int q = 0; q < 4; q++) {
-        float re[32], im[32];
-        tc_ld32(tl + q * 32, re);
-        tc_ld32(tl + TC_NROW + q * 32, im);
-        tc_wait_ld();
-        if (part == 0) {
-#pragma unroll
-            for (int i = 0; i < 32; i++)
-                tile[(q * 32 + i) * 64 + c] = make_float2(re[i], im[i]);
-        }
-        __syncthreads();
-        if (part == 1) {
-#pragma unroll
-            for (int i = 0; i < 32; i++) {
-                float2 v = tile[(q * 32 + i) * 64 + c];
-                v.x += re[i];
-                v.y += im[i];
-                if (a.fuse)
-                    v = cmul_nofma(v, a.kre, a.kim);
-                tile[(q * 32 + i) * 64 + c] = v;
-            }
-        }
-    }
-    tc_fence_before();
-    fence_proxy_async();
-    __syncthreads();
-    const long long left = a.n_out - m0;
-    const int count = left < TC_TILE ? (int)left : TC_TILE;
-    float2* dst = a.y + m0;
-    if (count == TC_TILE && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
-        if (tid == 0) {
-            asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(smem_u32(tile)),
-                         "r"((uint32_t)(TC_TILE * sizeof(float2)))
-                         : "memory");
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-        }
-    } else {
-        for (int i = tid; i < count; i += TC_THREADS)
-            dst[i] = tile[i];
-    }
-    if (warp == 0) {
-        __syncwarp();
-        tc_fence_after();
-        tc_dealloc(tmem, TC_TMEM_COLS);
-    }
-}
-
-// =================================================================================================
-// TF32 variant (algorithm 6): the same block-Toeplitz / Hankel-descriptor formulation with kind::tf32 operands,
-// built to MEASURE the second precision the tensor cores offer for this job (VERDICT r1, item 3), not to be fast:
-// decimation 1, one 4096-output tile per CTA, element-wise conversion.  A 128-byte swizzle row holds 32 tf32
-// values, so the Hankel shift is 32 samples and only 32 phases x {hi, lo} = 64 of the 128 tap rows carry data --
-// half of every MMA multiplies zeros -- K advances 8 per MMA instead of 16 and the tf32 pipe has half the bf16
-// rate: per useful product it costs ~8x the bf16 form, which is why the bf16 hi/lo split (3e-6 rel. RMS, inside
-// the 1e-5 bar) is the production form and this one (hi + lo carries 22 significand bits: ~1e-7) is not.
-constexpr int TF_PH = 32;
-constexpr int TF_TILE = TC_NROW * TF_PH;
-constexpr uint32_t TF_IDESC = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(TC_NROW >> 3) << 17) | ((128u >> 4) << 24);
-
-__device__ __forceinline__ void tc_mma_tf32(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate)
-{
-    asm volatile("{\n"
-                 ".reg .pred p;\n"
-                 "setp.ne.b32 p, %4, 0;\n"
-                 "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n"
-                 "}\n" ::"r"(d_tmem),
-                 "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-                 : "memory");
-}
-__device__ __forceinline__ float tf32_rna(float x)
-{
-    uint32_t u;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(u) : "f"(x));
-    return __uint_as_float(u);
-}
-__device__ __forceinline__ uint32_t tf_plane_off(uint32_t i)
-{
-    return (i >> 5) * 128u + ((((i >> 2) & 7u) ^ ((i >> 5) & 7u)) << 4) + (i & 3u) * 4u;
-}
-
-__global__ void __launch_bounds__(TC_THREADS, 2) fir_tc_tf32_kernel(const tc_args a)
-{
-    extern __shared__ uint8_t tc_smem_raw[];
-    uint8_t* smem = tc_align1024(tc_smem_raw);
-    uint8_t* planes = smem;                                   // [re_hi][re_lo][im_hi][im_lo], tf32 in fp32 containers
-    uint8_t* ring = smem + 4 * (size_t)a.plane_bytes;
-    uint64_t* bars = reinterpret_cast<uint64_t*>(ring + (size_t)a.stages * TC_ATOM_BYTES);
-    uint64_t* full = bars;
-    uint64_t* empty = bars + TC_MAX_STAGES;
-    uint64_t* done = bars + 2 * TC_MAX_STAGES;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * TC_MAX_STAGES + 1);
-    const int tid = threadIdx.x, warp = tc_warp_idx(), lane = tid & 31;
-    const long long m0 = (long long)blockIdx.x * TF_TILE;
-
-    if (tid == 0) {
-        for (int s = 0; s < a.stages; s++) {
-            mbar_init(&full[s], 1);
-            mbar_init(&empty[s], 1);
-        }
-        mbar_init(done, 1);
-        fence_mbar_init();
-    }
-    if (warp == 0) {
-        __syncwarp();
-        tc_alloc(tmem_slot, TC_TMEM_COLS);
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = *tmem_slot;
-
-    const long long j0 = m0 - a.P;
-    for (int i = tid; i < a.plane_elems; i += TC_THREADS) {
-        const long long n = j0 + i;
-        float2 v = make_float2(0.f, 0.f);
-        if (n >= 0) {
-            if (n < a.n_in)
-                v = __ldg(a.x + n);
-        } else if (a.hist != nullptr && n >= -(long long)a.Tm1) {
-            v = __ldg(a.hist + (a.Tm1 + n));
-        }
-        const float rh = tf32_rna(v.x), ih = tf32_rna(v.y);
-        const uint32_t off = tf_plane_off((uint32_t)i);
-        *reinterpret_cast<float*>(planes + off) = rh;
-        *reinterpret_cast<float*>(planes + a.plane_bytes + off) = tf32_rna(v.x - rh);
-        *reinterpret_cast<float*>(planes + 2 * a.plane_bytes + off) = ih;
-        *reinterpret_cast<float*>(planes + 3 * a.plane_bytes + off) = tf32_rna(v.y - ih);
-    }
-    fence_proxy_async();
-    __syncthreads();
-
-    if (warp == 0) {
-        const uint32_t planes_s = smem_u32(planes), ring_s = smem_u32(ring);
-        for (int at = 0; at < a.KA; at++) {
-            const int s = at % a.stages, use = at / a.stages;
-            if (at >= a.stages)
-                mbar_wait(&empty[s], (use & 1) ^ 1);
-            if (tc_elect_one()) {
-                mbar_arrive_expect_tx(&full[s], TC_ATOM_BYTES);
-                bulk_copy_g2s(ring + (size_t)s * TC_ATOM_BYTES, a.gA + (size_t)at * TC_ATOM_BYTES, TC_ATOM_BYTES, &full[s]);
-            }
-            __syncwarp();
-            mbar_wait(&full[s], use & 1);
-            tc_fence_after();
-            if (tc_elect_one()) {
-                const int nst = min(4, a.ksteps - 4 * at); // K-steps of 8 tf32 = 32 bytes
-                for (int t = 0; t < nst; t++) {
-                    const uint64_t adesc = tc_desc(ring_s + s * TC_ATOM_BYTES + t * 32, 0);
-                    const uint32_t boff = at * 128 + t * 32, acc = (at | t) != 0;
-                    tc_mma_tf32(tmem, adesc, tc_desc(planes_s + boff, 0), TF_IDESC, acc);
-                    tc_mma_tf32(tmem, adesc, tc_desc(planes_s + a.plane_bytes + boff, 0), TF_IDESC, 1);
-                    tc_mma_tf32(tmem + TC_NROW, adesc, tc_desc(planes_s + 2 * a.plane_bytes + boff, 0), TF_IDESC, acc);
-                    tc_mma_tf32(tmem + TC_NROW, adesc, tc_desc(planes_s + 3 * a.plane_bytes + boff, 0), TF_IDESC, 1);
-                }
-                tc_commit(&empty[s]);
-                if (at == a.KA - 1)
-                    tc_commit(done);
-            }
-            __syncwarp();
-        }
-    }
-    mbar_wait(done, 0);
-    tc_fence_after();
-
-    // lanes 0..31 (warp 0): hi-tap sums of phase c = lane, lanes 32..63 (warp 1): lo-tap sums; 64..127 are zero rows
-    float2* tile = reinterpret_cast<float2*>(planes);
-    const uint32_t tl = tmem + ((uint32_t)(warp * 32) << 16);
-#pragma unroll 1
-    for (int q = 0; q < 4; q++) {
-        float re[32], im[32];
-        tc_ld32(tl + q * 32, re);
-        tc_ld32(tl + TC_NROW + q * 32, im);
-        tc_wait_ld();
-        if (warp == 0) {
-#pragma unroll
-            for (int i = 0; i < 32; i++)
-                tile[(q * 32 + i) * TF_PH + lane] = make_float2(re[i], im[i]);
-        }
-        __syncthreads();
-        if (warp == 1) {
-#pragma unroll
-            for (int i = 0; i < 32; i++) {
-                float2 v = tile[(q * 32 + i) * TF_PH + lane];
-                v.x += re[i];
-                v.y += im[i];
-                if (a.fuse)
-                    v = cmul_nofma(v, a.kre, a.kim);
-                tile[(q * 32 + i) * TF_PH + lane] = v;
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    const long long left = a.n_out - m0;
-    const int count = left < TF_TILE ? (int)left : TF_TILE;
-    for (int i = tid; i < count; i += TC_THREADS)
-        a.y[m0 + i] = tile[i];
-    if (warp == 0) {
-        __syncwarp();
-        tc_fence_after();
-        tc_dealloc(tmem, TC_TMEM_COLS);
-    }
-}
 
 // =================================================================================================
 // Pipelined form: one persistent CTA per SM, warp-specialised.
@@ -469,8 +103,6 @@ template <int TCP_CONV, int TCP_LD>
 __device__ __forceinline__ void tc_convert(const tc_args& a, uint8_t* planes, int plane_elems, int plane_bytes,
                                            long long m0, int p, int ctid)
 {
-    if (a.dbg & 1)
-        return;
     const long long j0 = m0 - a.P;
     if (a.D == 1 && j0 >= 0 && j0 + plane_elems <= a.n_in && (reinterpret_cast<uintptr_t>(a.x) & 15) == 0) {
         // the whole tile (64-80 KB) is requested before the first conversion: TCP_LD independent 16-byte loads per thread
@@ -536,7 +168,7 @@ __device__ __forceinline__ void tc_convert(const tc_args& a, uint8_t* planes, in
     }
 }
 
-__global__ void __launch_bounds__(TCP_THREADS, 1) fir_tc_pipe_kernel(const tc_args a)
+__global__ void __launch_bounds__(TCP_THREADS, 1) fir_tc_pipe_kernel(const __grid_constant__ tc_args a)
 {
     extern __shared__ uint8_t tc_smem_raw[];
     uint8_t* smem = tc_align1024(tc_smem_raw);
@@ -601,10 +233,10 @@ __global__ void __launch_bounds__(TCP_THREADS, 1) fir_tc_pipe_kernel(const tc_ar
                     const int s = g % a.stages;
                     mbar_wait(&taps_full[s], (g / a.stages) & 1);
                     tc_fence_after();
-                    const int nst = (a.dbg & 4) ? 0 : min(4, a.ksteps - 4 * at);
+                    const int nst = min(4, a.ksteps - 4 * at);
                     if (tc_elect_one()) {
                         const uint64_t pstep = (uint64_t)(a.plane_bytes >> 4);
-                        uint64_t adesc = tc_desc(ring_s + s * TC_ATOM_BYTES, 0), b0 = tc_desc(pl + at * 128, 0);
+                        uint64_t adesc = tc_desc(ring_s + s * TC_ATOM_BYTES), b0 = tc_desc(pl + at * 128);
                         for (int t = 0; t < nst; t++, adesc += 2, b0 += 2) {
                             const uint32_t accum = (p | at | t) != 0;
                             tc_mma_bf16(d_re, adesc, b0, TC_IDESC, accum);
@@ -651,12 +283,6 @@ __global__ void __launch_bounds__(TCP_THREADS, 1) fir_tc_pipe_kernel(const tc_ar
             float2* dst = a.y + m0;
             mbar_wait(&tmem_full[acc], (it >> 1) & 1);
             tc_fence_after();
-            if (a.dbg & 2) {
-                __syncwarp();
-                if (lane == 0)
-                    mbar_arrive(&tmem_empty[acc]);
-                continue;
-            }
 #pragma unroll 1
             for (int q = 0; q < 4; q++, cq++) {
                 float re[32], im[32];
@@ -732,8 +358,8 @@ __global__ void __launch_bounds__(TCP_THREADS, 1) fir_tc_pipe_kernel(const tc_ar
 //   warps 4..11   epilogue: (warp & 3) = TMEM lane quarter, two warps per quarter split the 64 columns
 //                 (warps 4..7 also do the one-off tap upload into TMEM)
 //   warps 2, 3, 12..15  converters: staging (fp32) -> four swizzled bf16 planes, 3 plane stages
-// Measured on the way here (tools/tc_dbg.py, per 4096-sample tile and SM): with register-staged global
-// loads in the converters (two groups x 36 KB in flight) the conversion alone took 1.5 us and did not
+// Measured on the way here (roles switched off one at a time, per 4096-sample tile and SM): with register-staged
+// global loads in the converters (two groups x 36 KB in flight) the conversion alone took 1.5 us and did not
 // overlap the epilogue's stores (both latency-bound on the same memory system): 266 GS/s at 64 taps.
 constexpr int TS_NROW = 64;
 constexpr int TS_TILE = TS_NROW * TC_PH;  // 4096 outputs
@@ -764,8 +390,8 @@ template <bool REAL>
 __device__ __forceinline__ bool ts_head_tile(const tc_args& a, long long j0)
 {
     if (REAL)
-        return j0 == -(long long)a.P && a.P > 0 && ts_shift<REAL>(a) == 0 && 2 * TS_TILE <= a.n_in && !a.ts_nohead;
-    return j0 == -(long long)a.P && a.P > 0 && ts_shift<REAL>(a) == 0 && a.ts_plane_elems - a.P <= a.n_in && !a.ts_nohead;
+        return j0 == -(long long)a.P && a.P > 0 && ts_shift<REAL>(a) == 0 && 2 * TS_TILE <= a.n_in;
+    return j0 == -(long long)a.P && a.P > 0 && ts_shift<REAL>(a) == 0 && a.ts_plane_elems - a.P <= a.n_in;
 }
 // REAL: a tile's input is the 8192 + P floats from j0 on (run A: [j0, j0 + plane_elems), run B: 4096 further); the
 // bulk copies need a 16-byte aligned stream, j0 is a multiple of 16 samples
@@ -787,8 +413,6 @@ template <int NCONV>
 __device__ __forceinline__ void tc_convert_real(const tc_args& a, uint8_t* planes, int plane_elems, int plane_bytes,
                                                 long long m0, int ctid)
 {
-    if (a.dbg & 1)
-        return;
     const float* x = reinterpret_cast<const float*>(a.x);
     const float* hist = reinterpret_cast<const float*>(a.hist);
     const long long j0 = m0 - a.P;
@@ -824,7 +448,7 @@ __device__ __forceinline__ void tc_convert_real(const tc_args& a, uint8_t* plane
 }
 
 template <bool REAL>
-__global__ void __launch_bounds__(TS_THREADS, 1) fir_tc_ts_kernel(const tc_args a)
+__global__ void __launch_bounds__(TS_THREADS, 1) fir_tc_ts_kernel(const __grid_constant__ tc_args a)
 {
     extern __shared__ uint8_t tc_smem_raw[];
     uint8_t* smem = tc_align1024(tc_smem_raw);
@@ -881,12 +505,7 @@ __global__ void __launch_bounds__(TS_THREADS, 1) fir_tc_ts_kernel(const tc_args 
         for (int k = 0; k < a.ksteps; k++) {
             const uint4 lo4 = __ldg(reinterpret_cast<const uint4*>(row + k * 8));
             const uint4 hi4 = __ldg(reinterpret_cast<const uint4*>(row + k * 8 + 4));
-            uint32_t v[8] = { lo4.x, lo4.y, lo4.z, lo4.w, hi4.x, hi4.y, hi4.z, hi4.w };
-            if (a.ts_swap) {
-#pragma unroll
-                for (int i = 0; i < 8; i++)
-                    v[i] = __byte_perm(v[i], 0, 0x1032);
-            }
+            const uint32_t v[8] = { lo4.x, lo4.y, lo4.z, lo4.w, hi4.x, hi4.y, hi4.z, hi4.w };
             tc_st8(tl + k * 8, v);
         }
         asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
@@ -895,12 +514,10 @@ __global__ void __launch_bounds__(TS_THREADS, 1) fir_tc_ts_kernel(const tc_args 
     __syncthreads();
     tc_fence_after();
     const uint32_t d_base = tmem + TS_A_COLS;
-    if (a.ts_pdl) {
-        // programmatic dependent launch: everything above (barriers, TMEM, the tap upload) overlapped the tail of
-        // the previous kernel in the stream; nothing below may start before that kernel has completed and flushed
-        pdl_wait();
-        pdl_launch_dependents();
-    }
+    // programmatic dependent launch: everything above (barriers, TMEM, the tap upload) overlapped the tail of
+    // the previous kernel in the stream; nothing below may start before that kernel has completed and flushed
+    pdl_wait();
+    pdl_launch_dependents();
 
     if (warp == 0) {
         // ================= MMA issuer =================
@@ -912,12 +529,11 @@ __global__ void __launch_bounds__(TS_THREADS, 1) fir_tc_ts_kernel(const tc_args 
             tc_fence_after();
             const uint32_t d_re = d_base + acc * 2 * TS_NROW, d_im = d_re + TS_NROW;
             // descriptors of the four planes at K-step 0; a K-step advances the start address by 32 bytes = 2 units
-            uint64_t b0 = tc_desc(planes_s + ps * 4 * a.ts_plane_bytes, 0);
+            uint64_t b0 = tc_desc(planes_s + ps * 4 * a.ts_plane_bytes);
             const uint64_t pstep = (uint64_t)(a.ts_plane_bytes >> 4);
-            const int nk = (a.dbg & 4) ? 0 : a.ksteps;
             if (tc_elect_one()) {
 #pragma unroll 2
-                for (int k = 0; k < nk; k++, b0 += 2) {
+                for (int k = 0; k < a.ksteps; k++, b0 += 2) {
                     const uint32_t at = tmem + k * 8, accum = k != 0;
                     tc_mma_bf16_ts(d_re, at, b0, TS_IDESC, accum);
                     tc_mma_bf16_ts(d_re, at, b0 + pstep, TS_IDESC, 1);
@@ -973,12 +589,8 @@ __global__ void __launch_bounds__(TS_THREADS, 1) fir_tc_ts_kernel(const tc_args 
             } else if (lane == 0) {
                 const int sh = ts_shift<REAL>(a);
                 const uint32_t bytes = (uint32_t)(a.ts_plane_elems + 2 * sh) * 8u;
-                if (a.dbg & 8) {
-                    mbar_arrive(&in_full[slot]);
-                } else {
-                    mbar_arrive_expect_tx(&in_full[slot], bytes);
-                    bulk_copy_g2s(staging + (size_t)slot * a.ts_stage_bytes, a.x + j0 - sh, bytes, &in_full[slot]);
-                }
+                mbar_arrive_expect_tx(&in_full[slot], bytes);
+                bulk_copy_g2s(staging + (size_t)slot * a.ts_stage_bytes, a.x + j0 - sh, bytes, &in_full[slot]);
             }
             __syncwarp();
             nf++;
@@ -998,12 +610,6 @@ __global__ void __launch_bounds__(TS_THREADS, 1) fir_tc_ts_kernel(const tc_args 
             float* dstr = reinterpret_cast<float*>(a.y) + m0; // REAL: run A at dstr, run B 4096 floats further
             mbar_wait(&tmem_full[acc], (it >> 1) & 1);
             tc_fence_after();
-            if (a.dbg & 2) {
-                __syncwarp();
-                if (lane == 0)
-                    mbar_arrive(&tmem_empty[acc]);
-                continue;
-            }
             {
                 float re[32], im[32];
                 tc_ld32(tl + acc * 2 * TS_NROW + ch * 32, re);
@@ -1050,41 +656,39 @@ __global__ void __launch_bounds__(TS_THREADS, 1) fir_tc_ts_kernel(const tc_args 
             if (ts_fast_tile<REAL>(a, m0 - a.P)) {
                 const int slot = nf % TS_IN_STAGES;
                 mbar_wait(&in_full[slot], (nf / TS_IN_STAGES) & 1);
-                if (!(a.dbg & 1)) {
-                    const float2* src = reinterpret_cast<const float2*>(staging + (size_t)slot * a.ts_stage_bytes) + ts_shift<REAL>(a);
-                    const int npairs = a.ts_plane_elems >> 1;
-                    const bool al16 = ts_shift<REAL>(a) == 0;
+                const float2* src = reinterpret_cast<const float2*>(staging + (size_t)slot * a.ts_stage_bytes) + ts_shift<REAL>(a);
+                const int npairs = a.ts_plane_elems >> 1;
+                const bool al16 = ts_shift<REAL>(a) == 0;
 #pragma unroll 4
-                    for (int q = ctid; q < npairs; q += TS_CONV) {
-                        float4 v;
-                        if (REAL) {
-                            // samples 2q, 2q+1 of run A and of run B (4096 floats = 2048 float2 further)
-                            if (al16) {
-                                const float2* s2 = reinterpret_cast<const float2*>(staging + (size_t)slot * a.ts_stage_bytes);
-                                const float2 ra = s2[q], rb = s2[TS_TILE / 2 + q];
-                                v = make_float4(ra.x, rb.x, ra.y, rb.y);
-                            } else {
-                                const float* s1 = reinterpret_cast<const float*>(staging + (size_t)slot * a.ts_stage_bytes) +
-                                                  ts_shift<REAL>(a);
-                                v = make_float4(s1[2 * q], s1[TS_TILE + 2 * q], s1[2 * q + 1], s1[TS_TILE + 2 * q + 1]);
-                            }
-                        } else if (al16) {
-                            v = *reinterpret_cast<const float4*>(src + 2 * q);
+                for (int q = ctid; q < npairs; q += TS_CONV) {
+                    float4 v;
+                    if (REAL) {
+                        // samples 2q, 2q+1 of run A and of run B (4096 floats = 2048 float2 further)
+                        if (al16) {
+                            const float2* s2 = reinterpret_cast<const float2*>(staging + (size_t)slot * a.ts_stage_bytes);
+                            const float2 ra = s2[q], rb = s2[TS_TILE / 2 + q];
+                            v = make_float4(ra.x, rb.x, ra.y, rb.y);
                         } else {
-                            const float2 s0 = src[2 * q], s1 = src[2 * q + 1];
-                            v = make_float4(s0.x, s0.y, s1.x, s1.y);
+                            const float* s1 = reinterpret_cast<const float*>(staging + (size_t)slot * a.ts_stage_bytes) +
+                                              ts_shift<REAL>(a);
+                            v = make_float4(s1[2 * q], s1[TS_TILE + 2 * q], s1[2 * q + 1], s1[TS_TILE + 2 * q + 1]);
                         }
-                        const __nv_bfloat162 rh = __floats2bfloat162_rn(v.x, v.z);
-                        const __nv_bfloat162 ih = __floats2bfloat162_rn(v.y, v.w);
-                        const float2 rhf = __bfloat1622float2(rh), ihf = __bfloat1622float2(ih);
-                        const __nv_bfloat162 rl = __floats2bfloat162_rn(v.x - rhf.x, v.z - rhf.y);
-                        const __nv_bfloat162 il = __floats2bfloat162_rn(v.y - ihf.x, v.w - ihf.y);
-                        const uint32_t off = tc_plane_off(2u * q);
-                        *reinterpret_cast<__nv_bfloat162*>(pl + off) = rh;
-                        *reinterpret_cast<__nv_bfloat162*>(pl + a.ts_plane_bytes + off) = rl;
-                        *reinterpret_cast<__nv_bfloat162*>(pl + 2 * a.ts_plane_bytes + off) = ih;
-                        *reinterpret_cast<__nv_bfloat162*>(pl + 3 * a.ts_plane_bytes + off) = il;
+                    } else if (al16) {
+                        v = *reinterpret_cast<const float4*>(src + 2 * q);
+                    } else {
+                        const float2 s0 = src[2 * q], s1 = src[2 * q + 1];
+                        v = make_float4(s0.x, s0.y, s1.x, s1.y);
                     }
+                    const __nv_bfloat162 rh = __floats2bfloat162_rn(v.x, v.z);
+                    const __nv_bfloat162 ih = __floats2bfloat162_rn(v.y, v.w);
+                    const float2 rhf = __bfloat1622float2(rh), ihf = __bfloat1622float2(ih);
+                    const __nv_bfloat162 rl = __floats2bfloat162_rn(v.x - rhf.x, v.z - rhf.y);
+                    const __nv_bfloat162 il = __floats2bfloat162_rn(v.y - ihf.x, v.w - ihf.y);
+                    const uint32_t off = tc_plane_off(2u * q);
+                    *reinterpret_cast<__nv_bfloat162*>(pl + off) = rh;
+                    *reinterpret_cast<__nv_bfloat162*>(pl + a.ts_plane_bytes + off) = rl;
+                    *reinterpret_cast<__nv_bfloat162*>(pl + 2 * a.ts_plane_bytes + off) = ih;
+                    *reinterpret_cast<__nv_bfloat162*>(pl + 3 * a.ts_plane_bytes + off) = il;
                 }
                 __syncwarp();
                 if (lane == 0)
@@ -1112,19 +716,15 @@ __global__ void __launch_bounds__(TS_THREADS, 1) fir_tc_ts_kernel(const tc_args 
 
 // ---- host side ---------------------------------------------------------------------------------
 struct tc_plan {
-    int tf32 = 0;          // 1: TF32 measurement variant (fir_tc_tf32_kernel)
     int T = 0, D = 1;
-    int Tq = 0, P = 0, ksteps = 0, KA = 0, plane_elems = 0, plane_bytes = 0, stages = 2;
+    int Tq = 0, P = 0, ksteps = 0, KA = 0, plane_elems = 0, plane_bytes = 0;
     int fuse = 0;
     float kre = 1.f, kim = 0.f;
-    int desc_mode = 0;
-    size_t smem = 0;
     int real = 0;          // float stream (fff): tap-stationary kernel only
-    int ts = 0;            // 1: tap-stationary kernel (fir_tc_ts_kernel): D = 1, K <= 512
-    int ts_plane_elems = 0, ts_plane_bytes = 0, ts_stages = 0, ts_stage_bytes = 0, ts_swap = 0;
+    int ts = 0;            // 1: tap-stationary kernel (fir_tc_ts_kernel): D = 1, K <= 512; 0: ring form (fir_tc_pipe_kernel)
+    int ts_plane_elems = 0, ts_plane_bytes = 0, ts_stages = 0, ts_stage_bytes = 0;
     size_t ts_smem = 0;
     uint32_t* d_at = nullptr;
-    int pipe = 0;          // 1: persistent warp-specialised kernel (fir_tc_pipe_kernel)
     int pipe_stages = 2;
     size_t pipe_smem = 0;
     uint8_t* d_atoms = nullptr;
@@ -1157,66 +757,6 @@ bool tc_supported(int n_taps, int decimation, int real)
     return tq <= 2048;
 }
 
-static inline float tc_tf32_rna(float f)
-{
-    uint32_t u;
-    memcpy(&u, &f, 4);
-    u = (u + 0x1000u) & ~0x1fffu; // round to nearest, ties away, 10 explicit mantissa bits
-    memcpy(&f, &u, 4);
-    return f;
-}
-
-// TF32 measurement variant: decimation 1 only
-int tc_create_tf32(const float* taps, int n_taps, int fuse, float kre, float kim, tc_plan** out)
-{
-    *out = nullptr;
-    if (n_taps < 1 || n_taps > 2048)
-        return set_err(B200_ERR_UNSUPPORTED, "fir(tensor core, tf32): 1..2048 taps, decimation 1");
-    tc_plan* p = new tc_plan();
-    p->tf32 = 1;
-    p->T = n_taps;
-    p->D = 1;
-    p->Tq = n_taps;
-    p->P = (n_taps - 1 + 7) / 8 * 8;
-    const int kneed = p->P + TF_PH;
-    p->ksteps = kneed / 8;
-    p->KA = (kneed + 31) / 32;
-    p->plane_elems = TF_PH * (TC_NROW - 1) + kneed;
-    p->plane_bytes = ((p->plane_elems + 31) / 32 * 128 + 1023) / 1024 * 1024;
-    if (4 * p->plane_bytes < (int)(TF_TILE * sizeof(float2)))
-        p->plane_bytes = TF_TILE * sizeof(float2) / 4;
-    p->fuse = fuse;
-    p->kre = kre;
-    p->kim = kim;
-    p->stages = std::min(2, p->KA);
-    p->smem = 1024 + 4 * (size_t)p->plane_bytes + (size_t)p->stages * TC_ATOM_BYTES + 256;
-    std::vector<float> atoms((size_t)p->KA * TC_ATOM_BYTES / 4, 0.f);
-    for (int at = 0; at < p->KA; at++)
-        for (int row = 0; row < 64; row++) {
-            const int c = row & 31, lo = row >> 5;
-            for (int e = 0; e < 32; e++) {
-                const long long k = (long long)c + p->P - (32 * at + e);
-                const float hv = (k >= 0 && k < n_taps) ? taps[k] : 0.f;
-                const float hi = tc_tf32_rna(hv);
-                atoms[(size_t)at * (TC_ATOM_BYTES / 4) + (size_t)row * 32 + (size_t)(((e >> 2) ^ (row & 7)) << 2) + (e & 3)] =
-                    lo ? tc_tf32_rna(hv - hi) : hi;
-            }
-        }
-    cudaError_t e = cudaMalloc(&p->d_atoms, atoms.size() * 4);
-    if (e == cudaSuccess)
-        e = cudaMemcpy(p->d_atoms, atoms.data(), atoms.size() * 4, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(fir_tc_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess)
-        e = cudaDeviceSynchronize();
-    if (e != cudaSuccess) {
-        tc_destroy(p);
-        return set_err(B200_ERR_CUDA, "fir(tensor core, tf32) create: %s", cudaGetErrorString(e));
-    }
-    *out = p;
-    return B200_OK;
-}
-
 int tc_create(const float* taps, int n_taps, int decimation, int real, int fuse, float kre, float kim, tc_plan** out)
 {
     *out = nullptr;
@@ -1233,33 +773,12 @@ int tc_create(const float* taps, int n_taps, int decimation, int real, int fuse,
     p->KA = (kneed + 63) / 64;
     p->plane_elems = TC_PH * (TC_NROW - 1) + kneed;
     p->plane_bytes = ((p->plane_elems + 63) / 64 * 128 + 1023) / 1024 * 1024;
-    if (4 * p->plane_bytes < (int)(TC_TILE * sizeof(float2)))
-        p->plane_bytes = TC_TILE * sizeof(float2) / 4;
     p->fuse = fuse;
     p->kre = kre;
     p->kim = kim;
-    if (const char* e = getenv("B200_TC_DESC_MODE"))
-        p->desc_mode = atoi(e);
     const int total_atoms = p->D * p->KA;
-    // two CTAs per SM while the planes leave room for a 2-deep ring; a deeper ring when only one fits anyway
-    p->stages = 2;
-    size_t need = 1024 + 4 * (size_t)p->plane_bytes + 2 * TC_ATOM_BYTES + 256;
-    if (2 * need > 227 * 1024)
-        p->stages = TC_MAX_STAGES;
-    if (const char* e = getenv("B200_TC_STAGES"))
-        p->stages = atoi(e);
-    if (p->stages > TC_MAX_STAGES)
-        p->stages = TC_MAX_STAGES;
-    if (p->stages > total_atoms)
-        p->stages = total_atoms;
-    if (p->stages < 1)
-        p->stages = 1;
-    p->smem = 1024 + 4 * (size_t)p->plane_bytes + (size_t)p->stages * TC_ATOM_BYTES + 256;
-    if (p->smem > 227 * 1024) {
-        delete p;
-        return set_err(B200_ERR_UNSUPPORTED, "fir(tensor core): planes do not fit shared memory");
-    }
-    // pipelined form: two plane stages + the deepest tap ring that still fits
+    // ring form: two plane stages + the deepest tap ring that still fits.  At 2048 taps per branch a 2-deep ring
+    // needs 230 656 bytes, so every filter tc_supported accepts fits; the check guards that arithmetic.
     {
         const size_t fixed = 1024 + 8 * (size_t)p->plane_bytes + 2 * TCP_XBUF + 256;
         int st = TC_MAX_STAGES;
@@ -1269,9 +788,10 @@ int tc_create(const float* taps, int n_taps, int decimation, int real, int fuse,
             st = total_atoms;
         p->pipe_stages = st;
         p->pipe_smem = fixed + (size_t)st * TC_ATOM_BYTES;
-        p->pipe = p->pipe_smem <= 227 * 1024;
-        if (const char* e = getenv("B200_TC_PIPE"))
-            p->pipe = p->pipe && atoi(e) != 0;
+        if (p->pipe_smem > 227 * 1024) {
+            delete p;
+            return set_err(B200_ERR_UNSUPPORTED, "fir(tensor core): the tap ring does not fit shared memory");
+        }
     }
 
     // tap atoms: [branch][atom][row 0..127][64 bf16], rows 0..63 = hi part of phase c, 64..127 = lo part,
@@ -1317,21 +837,13 @@ int tc_create(const float* taps, int n_taps, int decimation, int real, int fuse,
         int st = TS_MAX_STAGES;
         while (st > 2 && 1024 + (size_t)st * 4 * p->ts_plane_bytes + (size_t)TS_IN_STAGES * p->ts_stage_bytes + 256 > 227 * 1024)
             st--;
-        if (const char* e = getenv("B200_TC_TS_STAGES"))
-            st = std::max(2, std::min(st, atoi(e)));
         p->ts_stages = st;
         p->ts_smem = 1024 + (size_t)st * 4 * p->ts_plane_bytes + (size_t)TS_IN_STAGES * p->ts_stage_bytes + 256;
         p->ts = 1;
-        if (const char* e = getenv("B200_TC_TS"))
-            p->ts = atoi(e) != 0 || p->real; // float streams exist in this kernel only
-        if (const char* e = getenv("B200_TC_TS_SWAP"))
-            p->ts_swap = atoi(e);
     }
     cudaError_t e = cudaMalloc(&p->d_atoms, atoms.size() * 2);
     if (e == cudaSuccess)
         e = cudaMemcpy(p->d_atoms, atoms.data(), atoms.size() * 2, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(fir_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e == cudaSuccess && !at_rows.empty()) {
         e = cudaMalloc(&p->d_at, at_rows.size() * 2);
         if (e == cudaSuccess)
@@ -1385,55 +897,27 @@ int tc_launch(tc_plan* p, const float* d_hist, const void* d_in, void* d_out, lo
     a.KA = p->KA;
     a.plane_elems = p->plane_elems;
     a.plane_bytes = p->plane_bytes;
-    a.stages = p->stages;
+    a.stages = p->pipe_stages;
     a.fuse = p->fuse;
     a.kre = p->kre;
     a.kim = p->kim;
-    a.desc_mode = p->desc_mode;
-    if (const char* e = getenv("B200_TC_DBG"))
-        a.dbg = atoi(e);
-    if (p->real && !p->ts)
-        return set_err(B200_ERR_UNSUPPORTED, "fir(tensor core): float streams need the tap-stationary kernel (<= 449 taps)");
-    if (p->tf32) {
-        const long long tf_tiles = (n_out + TF_TILE - 1) / TF_TILE;
-        B200_LAUNCH(fir_tc_tf32_kernel, (unsigned)tf_tiles, TC_THREADS, p->smem, s, a);
-        return B200_OK;
-    }
+    const long long sms = sm_count();
     if (p->ts) {
         a.gAt = p->d_at;
         a.ts_plane_elems = p->ts_plane_elems;
         a.ts_plane_bytes = p->ts_plane_bytes;
         a.ts_stages = p->ts_stages;
         a.ts_stage_bytes = p->ts_stage_bytes;
-        a.ts_swap = p->ts_swap;
         const long long tile_out = p->real ? 2 * TS_TILE : TS_TILE;
-        const long long ts_tiles = (n_out + tile_out - 1) / tile_out, sms = sm_count();
-        a.real = p->real;
-        static const int no_head = [] { const char* e = getenv("B200_TC_TS_HEAD"); return e && atoi(e) == 0; }();
-        static const int use_pdl = [] { const char* e = getenv("B200_TC_PDL"); return !e || atoi(e) != 0; }();
-        a.ts_nohead = no_head;
-        a.ts_pdl = use_pdl;
+        const long long ts_tiles = (n_out + tile_out - 1) / tile_out;
         const unsigned grid = (unsigned)(ts_tiles < sms ? ts_tiles : sms);
-        if (!use_pdl) {
-            if (p->real)
-                B200_LAUNCH(fir_tc_ts_kernel<true>, grid, TS_THREADS, p->ts_smem, s, a);
-            else
-                B200_LAUNCH(fir_tc_ts_kernel<false>, grid, TS_THREADS, p->ts_smem, s, a);
-            return B200_OK;
-        }
         if (p->real)
             B200_LAUNCH_PDL(fir_tc_ts_kernel<true>, grid, TS_THREADS, p->ts_smem, s, a);
         else
             B200_LAUNCH_PDL(fir_tc_ts_kernel<false>, grid, TS_THREADS, p->ts_smem, s, a);
         return B200_OK;
     }
-    if (p->pipe) {
-        a.stages = p->pipe_stages;
-        const long long sms = sm_count();
-        B200_LAUNCH(fir_tc_pipe_kernel, (unsigned)(tiles < sms ? tiles : sms), TCP_THREADS, p->pipe_smem, s, a);
-        return B200_OK;
-    }
-    B200_LAUNCH(fir_tc_kernel, (unsigned)tiles, TC_THREADS, p->smem, s, a);
+    B200_LAUNCH(fir_tc_pipe_kernel, (unsigned)(tiles < sms ? tiles : sms), TCP_THREADS, p->pipe_smem, s, a);
     return B200_OK;
 }
 

@@ -8,8 +8,6 @@ struct tc_plan;
 // decimation 1 and up to 449 taps (the tap-stationary kernel, two 4096-sample runs per tile)
 bool tc_supported(int n_taps, int decimation, int real);
 int tc_create(const float* taps, int n_taps, int decimation, int real, int fuse, float kre, float kim, tc_plan** out);
-// TF32 split, decimation 1: built to measure the second tensor-core precision (algorithm 6), not selected automatically
-int tc_create_tf32(const float* taps, int n_taps, int fuse, float kre, float kim, tc_plan** out);
 void tc_destroy(tc_plan* p);
 int tc_launch(tc_plan* p, const float* d_hist, const void* d_in, void* d_out, long long n_in,
               long long n_out, cudaStream_t s);

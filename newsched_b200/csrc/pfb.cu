@@ -459,8 +459,8 @@ __global__ void __launch_bounds__(PFBT_THREADS, 2)
             for (int ks = 0; ks < 8; ks++) {
                 // K-major: K-step = 32 bytes inside the 128-byte rows of a K-atom; MN-major: two 8-row atoms of 1 KiB
                 const uint32_t boff = mn ? ks * 2048 : (ks >> 2) * 8192 + (ks & 3) * 32;
-                const uint64_t bh = mn ? pfbt_desc_mn(planes_s + boff) : tc_desc(planes_s + boff, 0);
-                const uint64_t bl = mn ? pfbt_desc_mn(planes_s + PFBT_PLANE + boff) : tc_desc(planes_s + PFBT_PLANE + boff, 0);
+                const uint64_t bh = mn ? pfbt_desc_mn(planes_s + boff) : tc_desc(planes_s + boff);
+                const uint64_t bl = mn ? pfbt_desc_mn(planes_s + PFBT_PLANE + boff) : tc_desc(planes_s + PFBT_PLANE + boff);
                 tc_mma_bf16_ts_w(d, tmem + ks * 8, bh, idesc, ks != 0);   // F_hi u_hi
                 tc_mma_bf16_ts_w(d, tmem + 64 + ks * 8, bh, idesc, 1);    // F_lo u_hi
                 tc_mma_bf16_ts_w(d, tmem + ks * 8, bl, idesc, 1);         // F_hi u_lo

@@ -120,14 +120,12 @@ __device__ __forceinline__ void tc_ld32(uint32_t taddr, float (&v)[32])
 __device__ __forceinline__ void tc_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 // shared-memory matrix descriptor, K-major, SWIZZLE_128B: rows at 128 bytes, 8-row groups at SBO = 1024
-__device__ __forceinline__ uint64_t tc_desc(uint32_t saddr, int mode)
+__device__ __forceinline__ uint64_t tc_desc(uint32_t saddr)
 {
     uint64_t d = (uint64_t)((saddr >> 4) & 0x3FFF);
     d |= (uint64_t)1 << 16;            // leading byte offset (unused: a K-step lies inside one swizzle row)
     d |= (uint64_t)(1024 >> 4) << 32;  // stride byte offset between 8-row groups
     d |= (uint64_t)1 << 46;            // descriptor version (sm_100)
-    if (mode)
-        d |= (uint64_t)((saddr >> 7) & 7) << 49;
     d |= (uint64_t)2 << 61;            // SWIZZLE_128B
     return d;
 }

@@ -438,66 +438,6 @@ def test_interp_fir_impulse_exact_and_empty(cuda):
         nb.RationalResampler(taps, 1, 5000)      # plain heavy decimation belongs to fir_filter
 
 
-@pytest.mark.parametrize("T,cplxin", [(4, True), (31, True), (32, True), (48, True), (64, True), (65, True),
-                                      (95, True), (128, True), (500, True), (2048, True),
-                                      (5, False), (64, False), (100, False), (129, False), (1000, False)])
-def test_fir_two_parallel_form(cuda, T, cplxin):
-    """algorithm 5 (2-parallel fast FIR, 0.77x the FMAs of the direct form): within tolerance of the
-    fp64 oracle and of the direct form; bit-identical when the stream is cut or segmented at even
-    offsets."""
-    import newsched_b200 as nb
-    rng = np.random.default_rng(T * 5 + cplxin)
-    n = 3 * 4096 * 5 + 1235
-    x = cplx(rng, n) if cplxin else rng.uniform(-1, 1, n).astype(np.float32)
-    taps = (rng.uniform(-1, 1, T) / T).astype(np.float32)
-    dx = dev(cuda, x)
-    f = nb.FirFilter(taps, 1, is_complex=cplxin, algorithm=5)
-    assert f.algorithm == 5
-    y, nc = f.work(dx)
-    ref = o.fir(x, taps, 1)
-    assert y.numel() == n and nc == n
-    assert o.rel_rms(host(y), ref) < TOL_RMS
-    assert np.max(np.abs(host(y) - ref)) < 1e-4 * np.max(np.abs(ref))
-    yd, _ = nb.FirFilter(taps, 1, is_complex=cplxin, algorithm=1).work(dx)
-    assert o.rel_rms(host(y), host(yd)) < TOL_RMS
-    one = host(y)
-    # streaming: even cut points reproduce the one-shot bits (an output's arithmetic depends only on
-    # the parity of its index within the call); odd cuts stay within tolerance
-    for chunks, exact in (((5000, 2, 4096, 33334, 8, 10 ** 9), True), ((5001, 1, 4096, 33333, 7, 10 ** 9), False)):
-        f2 = nb.FirFilter(taps, 1, is_complex=cplxin, algorithm=5)
-        outs, pos = [], 0
-        for chunk in chunks:
-            if pos >= n:
-                break
-            yy, c = f2.work(dx[pos:min(pos + chunk, n)])
-            outs.append(host(yy))
-            pos += c
-        got = np.concatenate(outs)
-        assert got.size == n
-        if exact:
-            assert np.array_equal(got, one), "chunked at even offsets != one-shot"
-        else:
-            assert o.rel_rms(got, ref) < TOL_RMS
-    if T > 1:
-        L = (n // 3) // 2 * 2
-        parts = []
-        for g in range(3):
-            lo, hi = g * L, (n if g == 2 else (g + 1) * L)
-            halo = None if g == 0 else dx[lo - (T - 1):lo]
-            parts.append(host(f.work_segment(dx[lo:hi], halo)))
-        assert np.array_equal(np.concatenate(parts), one), "time segments + halo != one stream"
-    k = 0.5 - 0.25j if cplxin else 3.25
-    yk, _ = nb.FirFilter(taps, 1, is_complex=cplxin, multiply_const=k, algorithm=5).work(dx)
-    if cplxin:
-        assert np.array_equal(host(yk), o.multiply_const(one, k)), "fused epilogue != two-block chain"
-    else:
-        assert np.array_equal(host(yk), one * np.float32(k))
-    # output pointer not 16-byte aligned: the TMA store is replaced by the plain store loop
-    buf = cuda.zeros(n + 1, dtype=dx.dtype, device="cuda")
-    f.work_segment(dx, None, buf[1:])
-    assert np.array_equal(host(buf[1:]), one) and buf[0].item() == 0
-
-
 @pytest.mark.parametrize("T,D,cplxin", [(16, 2, True), (64, 2, True), (96, 4, True), (160, 4, True), (33, 8, True),
                                         (192, 8, True), (64, 16, True), (384, 16, True), (64, 2, False),
                                         (256, 4, False), (100, 8, False), (500, 16, False), (64, 32, False),
@@ -664,6 +604,14 @@ def test_fir_tensor_core_form_rejects_what_it_cannot_do(cuda):
         nb.FirFilter(np.ones(450, np.float32), 1, is_complex=False, algorithm=2)   # ... and taps resident in TMEM (K <= 512)
     with pytest.raises(nb.B200Error):
         nb.FirFilter(np.ones(64, np.float32), 9, algorithm=2)                      # decimation > 8
+
+
+@pytest.mark.parametrize("algorithm", [-1, 5, 6, 7])
+def test_fir_rejects_unknown_algorithm(cuda, algorithm):
+    """algorithm is 0 (auto) or one of the forms 1..4; any other value is an error, not a silent direct form."""
+    import newsched_b200 as nb
+    with pytest.raises(nb.B200Error, match="algorithm must be"):
+        nb.FirFilter(np.ones(64, np.float32), 1, algorithm=algorithm)
 
 
 @pytest.mark.parametrize("T", [33, 64, 100, 256, 448, 5])

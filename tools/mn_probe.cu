@@ -73,10 +73,10 @@ __global__ void __launch_bounds__(128, 1) mn_probe_kernel(const uint16_t* gA, co
         if (mode != 2)
             idesc |= 1u << 16;
         for (int s = 0; s < 4; s++) {
-            const uint64_t ad = tc_desc(smem_u32(sA) + s * 32, 0);
+            const uint64_t ad = tc_desc(smem_u32(sA) + s * 32);
             uint64_t bd;
             if (mode == 2)
-                bd = tc_desc(smem_u32(sB) + s * 32, 0);
+                bd = tc_desc(smem_u32(sB) + s * 32);
             else if (mode == 0)
                 bd = probe_desc(smem_u32(sB) + s * 2048, 8192, 1024);
             else

@@ -1,5 +1,5 @@
 """Runs one hot-path kernel a few times on synthetic data (for ncu captures / launch lists).
-usage: python tools/prof_one.py fftmag|fft|fftnN|tcT|fir64simt|fir64|firdec64d4|firdec64d5|rs32|fir1024d4|fir4096|ffa64|pfb|pfbtc|pfb16|copy [reps]"""
+usage: python tools/prof_one.py fftmag|fft|fftnN|tcT|fir64simt|fir64|firdec64d4|firdec64d5|rs32|fir1024d4|fir4096|pfb|pfbtc|pfb16|copy [reps]"""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -30,8 +30,6 @@ elif what.startswith("tc"):          # tensor-core (tcgen05) FIR, e.g. tc64 / tc
     op = nb.FirFilter((rng.uniform(-1, 1, T) / T).astype(np.float32), algorithm=2); out = torch.empty_like(x); fn = lambda: op.work_segment(x, None, out)
 elif what == "fir64simt":
     op = nb.FirFilter((rng.uniform(-1, 1, 64) / 64).astype(np.float32), algorithm=1); out = torch.empty_like(x); fn = lambda: op.work_segment(x, None, out)
-elif what == "ffa64":
-    op = nb.FirFilter((rng.uniform(-1, 1, 64) / 64).astype(np.float32), algorithm=5); out = torch.empty_like(x); fn = lambda: op.work_segment(x, None, out)
 elif what == "firdec64d4":
     n = N * 32768; x = torch.view_as_complex(torch.rand(n, 2, device="cuda", generator=g) * 2 - 1)
     op = nb.FirFilter((rng.uniform(-1, 1, 64) / 64).astype(np.float32), 4); out = torch.empty(n // 4, dtype=torch.complex64, device="cuda"); fn = lambda: op.work_segment(x, None, out)

@@ -219,11 +219,25 @@ B200_API int b200_fft_destroy(b200_fft* h);
 B200_API int b200_fft_run(b200_fft* h, const void* d_in, void* d_out, int64_t n_vectors, b200_stream_t s);
 B200_API int b200_fft_geometry(const b200_fft* h, int* n, int* out_item_bytes);
 
-/* ---- polyphase channelizer (critically sampled analysis bank, M channels) ----------
+/* ---- polyphase channelizer (analysis bank, M channels, critically sampled or oversampled) ----------
  * SURVEY.md 8(c): taps h[0..M*P), u_i[t] = sum_r h[i+rM] x[(t-r)M + M-1-i],
  * y_c[t] = sum_i u_i[t] e^{+j 2 pi i c / M}; out[t*M + c].  Handle keeps (P-1)*M history.
  * channel_begin/channel_count select a slice of output channels (channel sharding);
- * out is then [t][channel_count]. */
+ * out is then [t][channel_count].
+ *
+ * oversample OS = 2 or 4 (GNU Radio's pfb_channelizer_ccf oversample_rate): one frame per hop D = M/OS input
+ * samples, so adjacent channels overlap and a signal on a channel boundary is whole in both.  With t the frame
+ * index since creation or the last reset (input before the stream start is zero):
+ *   z_c[t] = e^{-j 2 pi c tD/M} sum_{n<MP} h[n] e^{+j 2 pi n c/M} x[tD + D-1-n]
+ *          = sum_{i<M} u_{(i + tD) mod M}[t] e^{+j 2 pi i c/M},  u_i[t] = sum_r h[i+rM] x[tD + D-1-i-rM]
+ * Every channel is at baseband (a tone at c0 fs/M is a constant phasor in channel c0).  OS = 1 is the formula
+ * above.  A run consumes n_frames*D items and produces n_frames = floor(n_in/D) vectors; the handle keeps the
+ * last P*M - D input samples and the frame phase (frames produced mod OS); b200_pfb_reset zeroes both.
+ * b200_pfb_run_segment is stateless: d_halo holds the P*M - D samples before d_in (NULL = zeros) and d_in[0]
+ * starts frame phase 0, so segments meant to join into one stream must start at multiples of M input samples
+ * (e.g. multigpu.time_segments(..., align=M)).
+ * OS > 1 needs M in 16..256 and the single-pass kernel (P up to its shared-memory limit; B200_ERR_UNSUPPORTED
+ * otherwise), and the SIMT DFT (algorithm 2 is refused with B200_ERR_UNSUPPORTED). */
 typedef struct b200_pfb b200_pfb;
 typedef struct {
     const float* taps;   /* host, M*P floats */
@@ -231,6 +245,7 @@ typedef struct {
     int32_t taps_per_channel; /* P */
     int32_t channel_begin;
     int32_t channel_count; /* 0 = all */
+    int32_t oversample;    /* 0 or 1 = critically sampled; 2, 4 = oversampled; anything else: B200_ERR_ARG */
 } b200_pfb_params;
 B200_API int b200_pfb_create(const b200_pfb_params* p, b200_pfb** h);
 B200_API int b200_pfb_destroy(b200_pfb* h);
@@ -247,6 +262,7 @@ B200_API int b200_pfb_geometry(const b200_pfb* h, int* n_channels, int* channel_
  *       channel; B200_ERR_UNSUPPORTED otherwise).  Same results within the 1e-5 relative-RMS bar. */
 B200_API int b200_pfb_set_algorithm(b200_pfb* h, int32_t algorithm);
 B200_API int b200_pfb_get_algorithm(const b200_pfb* h, int32_t* algorithm);
+B200_API int b200_pfb_get_oversample(const b200_pfb* h, int32_t* oversample); /* 1, 2 or 4 */
 
 /* ---- host-buffer streaming driver (the e2e path a host-resident source/sink sees) ---
  * A chain is an ordered list of op handles executed back to back on device buffers; the

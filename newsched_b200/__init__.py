@@ -60,7 +60,7 @@ class _FftParams(C.Structure):
 class _PfbParams(C.Structure):
     _fields_ = [("taps", C.POINTER(C.c_float)), ("n_channels", C.c_int32),
                 ("taps_per_channel", C.c_int32), ("channel_begin", C.c_int32),
-                ("channel_count", C.c_int32)]
+                ("channel_count", C.c_int32), ("oversample", C.c_int32)]
 
 
 class IpcHandle(C.Structure):
@@ -157,6 +157,7 @@ SIGNATURES = {
     "b200_pfb_geometry": (_I, [_V, C.POINTER(_I), C.POINTER(_I)]),
     "b200_pfb_set_algorithm": (_I, [_V, C.c_int32]),
     "b200_pfb_get_algorithm": (_I, [_V, C.POINTER(C.c_int32)]),
+    "b200_pfb_get_oversample": (_I, [_V, C.POINTER(C.c_int32)]),
     "b200_chain_create": (_I, [C.POINTER(_ChainOp), C.c_int32, C.c_int32, _I64, C.POINTER(_V)]),
     "b200_chain_destroy": (_I, [_V]),
     "b200_chain_run": (_I, [_V, _V, _V, _I64, _PI64, _V]),
@@ -529,14 +530,17 @@ class RationalResampler:
 
 
 class PfbChannelizer:
-    """Critically sampled M-channel polyphase analysis bank; work() returns [n_t, channels]."""
+    """M-channel polyphase analysis bank, one output frame per hop = M / oversample input items;
+    work() returns [n_t, channels]."""
 
     def __init__(self, taps, n_channels: int, channel_begin: int = 0, channel_count: int = 0,
-                 algorithm: int = 0):
-        """algorithm: 0 auto, 1 SIMT DFT, 2 DFT across branches as a tensor-core GEMM (64 channels only)."""
+                 algorithm: int = 0, oversample: int = 1):
+        """algorithm: 0 auto, 1 SIMT DFT, 2 DFT across branches as a tensor-core GEMM (64 channels only).
+        oversample: 1 critically sampled, 2 or 4 (M = 16 .. 256; see b200_pfb_params in include/b200dsp.h)."""
         arr, ptr = _floats(taps)
         assert arr.size % n_channels == 0
-        p = _PfbParams(ptr, int(n_channels), arr.size // n_channels, int(channel_begin), int(channel_count))
+        p = _PfbParams(ptr, int(n_channels), arr.size // n_channels, int(channel_begin), int(channel_count),
+                       int(oversample))
         h = C.c_void_p()
         _check(lib().b200_pfb_create(C.byref(p), C.byref(h)))
         self._h = h
@@ -550,6 +554,8 @@ class PfbChannelizer:
         self.m = int(n_channels)
         self.p = arr.size // n_channels
         self.channels = int(channel_count) if channel_count else self.m - int(channel_begin)
+        self.oversample = self._get_oversample()
+        self.hop = self.m // self.oversample
 
     @property
     def handle(self):
@@ -561,11 +567,16 @@ class PfbChannelizer:
         _check(lib().b200_pfb_get_algorithm(self._h, C.byref(a)))
         return a.value
 
+    def _get_oversample(self) -> int:
+        v = C.c_int32()
+        _check(lib().b200_pfb_get_oversample(self._h, C.byref(v)))
+        return v.value
+
     def work(self, x, out=None, stream=None):
         torch = _torch()
         _need_cuda(x)
         assert x.dtype == torch.complex64
-        n_t = x.numel() // self.m
+        n_t = x.numel() // self.hop
         if out is None:
             out = torch.empty((n_t, self.channels), dtype=torch.complex64, device=x.device)
         else:
@@ -579,13 +590,13 @@ class PfbChannelizer:
         torch = _torch()
         _need_cuda(x)
         assert x.dtype == torch.complex64
-        n_t = x.numel() // self.m
+        n_t = x.numel() // self.hop
         if out is None:
             out = torch.empty((n_t, self.channels), dtype=torch.complex64, device=x.device)
         else:
             _need_out(out, x, n_t * self.channels)
         nv = C.c_int64()
-        _check(lib().b200_pfb_run_segment(self._h, _halo_ptr(halo, x, (self.p - 1) * self.m),
+        _check(lib().b200_pfb_run_segment(self._h, _halo_ptr(halo, x, self.p * self.m - self.hop),
                                           x.data_ptr(), out.data_ptr(), x.numel(), C.byref(nv),
                                           _stream(stream)))
         return out[: nv.value]

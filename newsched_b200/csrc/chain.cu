@@ -182,14 +182,17 @@ int b200_chain_create(const b200_chain_op* ops, int32_t n_ops, int32_t in_item_b
             st.multiple = n;
         } else if (st.op.kind == B200_OP_PFB) {
             int m = 0, cc = 0;
+            int32_t os = 1;
             rc = b200_pfb_geometry((b200_pfb*)st.op.handle, &m, &cc);
+            if (rc == B200_OK)
+                rc = b200_pfb_get_oversample((b200_pfb*)st.op.handle, &os);
             if (rc == B200_OK && bytes != 8)
                 rc = set_err(B200_ERR_ARG, "chain: pfb needs complex64 items");
             st.in_item_bytes = 8;
             st.out_item_bytes = 8;
-            st.num = cc;
-            st.den = m;
-            st.multiple = m;
+            st.num = cc; // cc channels out per hop of D = M / oversample items in
+            st.den = m / os;
+            st.multiple = m / os;
         } else {
             rc = stage_describe(st, bytes);
         }

@@ -98,21 +98,25 @@ constexpr int PFB64_RS = 68;  // u row stride (complex): 68 = 4 mod 16 keeps the
 // The input tile is one contiguous span of the stream, so interior tiles are staged by a 1-D TMA
 // bulk copy issued as soon as the branch filters of the previous tile have consumed X -- it lands
 // while the 64-point DFTs and the output stores of that tile run.
-template <int P4T> // > 0: taps per branch known at compile time (fully unrolled filters)
+// OS = 2, 4 (oversampled bank, DESIGN.md 4.4e): frames advance by D = 64 / OS samples, the input tile is
+// TT + P4 OS - 1 rows of D samples, and branch outputs go to their circularly shifted U slot.
+template <int P4T, int OS = 1> // P4T > 0: taps per branch known at compile time (fully unrolled filters)
 __global__ void __launch_bounds__(256, 2)
     pfb64_kernel(const float2* __restrict__ x, const float2* __restrict__ halo, float2* __restrict__ out,
                  const float* __restrict__ taps_rm /* [P4][64] */, int P4, int Ptrue,
-                 long long n_frames, long long n_in, int ch_begin, int ch_count, int tma_ok, int nbuf)
+                 long long n_frames, long long n_in, int ch_begin, int ch_count, int tma_ok, int nbuf,
+                 int phase0 /* OS > 1: (frame index of out[0]) mod OS */)
 {
+    constexpr int D = 64 / OS; // hop: input samples per frame = samples per row of the input tile
     // nbuf = 2 (P4T > 0 and P <= 16, see b200_pfb_create): TWO input tiles, the copy of tile i+1 is issued a whole tile
     // ahead of its use.  With one buffer the copy only had the DFT stage to hide behind and 10.5 % of all warp samples
     // sat on the input mbarrier (ncu r02_pfb64_v4).  Two tiles + U are exactly the 115 712 bytes a CTA may use with two
     // CTAs per SM, so the taps live in registers for the lifetime of the CTA (no shared copy) and the two mbarriers sit
     // in the padding of U's first row (elements 64..67 of a row are never touched).
     extern __shared__ __align__(128) float2 sm[];
-    const int rows = PFB64_TT + P4 - 1;
+    const int rows = PFB64_TT + P4 * OS - 1;
     float2* X0 = sm;
-    float2* U = X0 + nbuf * rows * 64;
+    float2* U = X0 + nbuf * rows * D;
     uint64_t* bar = reinterpret_cast<uint64_t*>(U + 64);
     float* hT = reinterpret_cast<float*>(U + PFB64_TT * PFB64_RS); // only when P4T == 0 (taps not in registers)
     const int tid = threadIdx.x;
@@ -130,7 +134,7 @@ __global__ void __launch_bounds__(256, 2)
         for (int r = 0; r < P4T; r++)
             hreg[r] = __ldg(taps_rm + r * 64 + (tid & 63));
     }
-    const long long nh = (long long)(Ptrue - 1) * 64;
+    const long long nh = (long long)(Ptrue - 1) * 64 + (64 - D); // P M - D samples of history
     const long long n_tiles = (n_frames + PFB64_TT - 1) / PFB64_TT;
     // stage-1 twiddles W64^{i0 c1} depend on the thread only (i0 = tid & 3): register resident
     float2 twr[16];
@@ -140,11 +144,11 @@ __global__ void __launch_bounds__(256, 2)
         sincospif((float)(((tid & 3) * c1) & 63) / 32.0f, &sn, &cs_); // e^{+j 2 pi i0 c1 / 64}
         twr[c1] = make_float2(cs_, sn);
     }
-    const uint32_t tile_bytes = (uint32_t)rows * 64u * 8u;
+    const uint32_t tile_bytes = (uint32_t)rows * (uint32_t)D * 8u;
     // can tile `t` be staged by TMA?  (whole span inside [0, n_in), 16-byte aligned source)
     auto tma_tile = [&](long long t) {
-        const long long g0 = (t * PFB64_TT - (P4 - 1)) * 64;
-        return tma_ok && g0 >= 0 && g0 + (long long)rows * 64 <= n_in;
+        const long long g0 = (t * PFB64_TT - (P4 * OS - 1)) * D;
+        return tma_ok && g0 >= 0 && g0 + (long long)rows * D <= n_in;
     };
     __syncthreads();
     // programmatic dependent launch (B200_LAUNCH_PDL): the prologue above ran while the previous kernel in the
@@ -157,7 +161,7 @@ __global__ void __launch_bounds__(256, 2)
             const long long t = tile + (long long)b * gridDim.x;
             if (t < n_tiles && tma_tile(t)) {
                 mbar_arrive_expect_tx(bar + b, tile_bytes);
-                bulk_copy_g2s(X0 + b * rows * 64, x + (t * PFB64_TT - (P4 - 1)) * 64, tile_bytes, bar + b);
+                bulk_copy_g2s(X0 + b * rows * D, x + (t * PFB64_TT - (P4 * OS - 1)) * D, tile_bytes, bar + b);
             }
         }
     uint32_t phase = 0; // bit b: parity of the next completion of bar[b]
@@ -166,22 +170,22 @@ __global__ void __launch_bounds__(256, 2)
     for (; tile < n_tiles; tile += gridDim.x, it++) {
         const long long f0 = tile * PFB64_TT; // first frame of the tile
         const int xb = nbuf == 2 ? (it & 1) : 0;
-        float2* X = X0 + xb * rows * 64;
-        // rows: row j holds frame (f0 - (P4-1) + j), col = position within the frame
+        float2* X = X0 + xb * rows * D;
+        // rows: row j holds samples [(f0 - (P4 OS - 1) + j) D, ... + D); at OS = 1 frame (f0 - (P4-1) + j)
         if (tma_tile(tile)) {
             mbar_wait(bar + xb, (phase >> xb) & 1u);
             phase ^= 1u << xb;
         } else {
-            const long long g0 = (f0 - (P4 - 1)) * 64;
-            for (int i0 = tid; i0 < rows * 64; i0 += 256 * 8) {
+            const long long g0 = (f0 - (P4 * OS - 1)) * D;
+            for (int i0 = tid; i0 < rows * D; i0 += 256 * 8) {
                 float2 v[8];
 #pragma unroll
                 for (int u = 0; u < 8; u++)
-                    if (i0 + u * 256 < rows * 64)
+                    if (i0 + u * 256 < rows * D)
                         v[u] = pfb_fetch(x, halo, nh, g0 + i0 + u * 256, n_in);
 #pragma unroll
                 for (int u = 0; u < 8; u++)
-                    if (i0 + u * 256 < rows * 64)
+                    if (i0 + u * 256 < rows * D)
                         X[i0 + u * 256] = v[u];
             }
             __syncthreads();
@@ -190,53 +194,58 @@ __global__ void __launch_bounds__(256, 2)
         // ---- branch filters: thread = (branch i, 16 consecutive frames) ------------------
         {
             const int i = tid & 63, tg = tid >> 6;
-            const float2* col = X + (63 - i) + (tg * 16) * 64; // row (tg*16 + j + (P4-1) - r)
+            // branch i = a D + b, frame j of the thread, tap r: column D-1-b of row tg*16 + j + (P4-1-r) OS + (OS-1-a)
+            // (OS = 1: a = 0, b = i, row tg*16 + j + (P4-1) - r)
+            const int a = i / D, b = i % D;
+            const float2* col = X + (D - 1 - b) + (tg * 16 + OS - 1 - a) * D;
             float2 acc[16];
 #pragma unroll
             for (int j = 0; j < 16; j++)
                 acc[j] = make_float2(0.f, 0.f);
             if (P4T > 0) {
                 // taps in registers, every input row read exactly once: row rho feeds the
-                // (frame j, tap r) pairs with j + P4-1 - r == rho
+                // (frame j, tap r) pairs with j + (P4-1 - r) OS == rho
 #pragma unroll
-                for (int rho = 0; rho < 16 + P4T - 1; rho++) {
-                    const float2 v = col[rho * 64];
+                for (int rho = 0; rho < 16 + (P4T - 1) * OS; rho++) {
+                    const float2 v = col[rho * D];
 #pragma unroll
                     for (int j = 0; j < 16; j++) {
-                        const int r = j + P4T - 1 - rho;
-                        if (r >= 0 && r < P4T)
+                        const int r = P4T - 1 - (rho - j) / OS;
+                        if ((rho - j) % OS == 0 && r >= 0 && r < P4T)
                             acc[j] = __ffma2_rn(v, make_float2(hreg[r], hreg[r]), acc[j]);
                     }
                 }
             } else {
                 for (int rc = 0; rc < P4; rc += 4) {
-                    // taps r = rc..rc+3 ; rows needed: j + (P4-1) - r for j in 0..15
+                    // taps r = rc..rc+3 ; rows needed: j + (P4-1 - r) OS for j in 0..15
                     const float h0 = hT[(rc + 0) * 64 + i], h1 = hT[(rc + 1) * 64 + i];
                     const float h2 = hT[(rc + 2) * 64 + i], h3 = hT[(rc + 3) * 64 + i];
-                    const float2* base = col + (P4 - 1 - rc - 3) * 64;
-                    float2 w[19];
+                    const float2* base = col + (P4 - 1 - rc - 3) * OS * D;
+                    float2 w[16 + 3 * OS];
 #pragma unroll
-                    for (int q = 0; q < 19; q++)
-                        w[q] = base[q * 64];
+                    for (int q = 0; q < 16 + 3 * OS; q++)
+                        w[q] = base[q * D];
 #pragma unroll
                     for (int j = 0; j < 16; j++) {
-                        acc[j] = __ffma2_rn(w[j + 3], make_float2(h0, h0), acc[j]);
-                        acc[j] = __ffma2_rn(w[j + 2], make_float2(h1, h1), acc[j]);
-                        acc[j] = __ffma2_rn(w[j + 1], make_float2(h2, h2), acc[j]);
+                        acc[j] = __ffma2_rn(w[j + 3 * OS], make_float2(h0, h0), acc[j]);
+                        acc[j] = __ffma2_rn(w[j + 2 * OS], make_float2(h1, h1), acc[j]);
+                        acc[j] = __ffma2_rn(w[j + OS], make_float2(h2, h2), acc[j]);
                         acc[j] = __ffma2_rn(w[j], make_float2(h3, h3), acc[j]);
                     }
                 }
             }
+            // circular shift of the branches: u_i[t] goes to slot (i - t D) mod 64, t = phase0 + f0 + tg*16 + j, and
+            // f0 + tg*16 is a multiple of OS.  Consecutive lanes still write a contiguous run (mod 64) of a row.
 #pragma unroll
             for (int j = 0; j < 16; j++)
-                U[(tg * 16 + j) * PFB64_RS + i] = acc[j];
+                U[(tg * 16 + j) * PFB64_RS + (OS == 1 ? i : (i - (phase0 + j) * D) & 63)] = acc[j];
         }
         __syncthreads(); // U complete; X fully consumed
         {
             const long long nxt = tile + (long long)nbuf * gridDim.x; // refill the buffer just consumed
             if (tid == 0 && nxt < n_tiles && tma_tile(nxt)) {
                 mbar_arrive_expect_tx(bar + xb, tile_bytes);
-                bulk_copy_g2s(X, x + (nxt * PFB64_TT - (P4 - 1)) * 64, tile_bytes, bar + xb);
+                bulk_copy_g2s(X, x + (nxt * PFB64_TT - (P4 * OS - 1)) * D, tile_bytes, bar + xb);
             }
         }
 
@@ -615,20 +624,22 @@ __device__ __forceinline__ void idft8(float2 (&z)[8])
     z[3] = f2add(e3, o3), z[7] = f2sub(e3, o3);
 }
 
-template <int M, int P4T>
+// OS = 2, 4: oversampled bank, the same changes as pfb64_kernel (rows of D = M / OS samples, shifted U slots).
+template <int M, int P4T, int OS = 1>
 __global__ void __launch_bounds__(256, (M >= 128 ? 1 : 2))
     pfbm_kernel(const float2* __restrict__ x, const float2* __restrict__ halo, float2* __restrict__ out,
                 const float* __restrict__ taps_rm /* [P4][M] */, int P4, int Ptrue, long long n_frames,
-                long long n_in, int ch_begin, int ch_count, int tma_ok, int nbuf)
+                long long n_in, int ch_begin, int ch_count, int tma_ok, int nbuf,
+                int phase0 /* OS > 1: (frame index of out[0]) mod OS */)
 {
     // nbuf = 2 (when shared memory allows, see b200_pfb_create): two input tiles, the copy of tile i+1 is issued a
     // whole tile ahead.  With one buffer it only had the DFT stage to hide behind: M = 128 (one CTA per SM) spent
     // 17 % of its warp samples on the input mbarrier (ncu, round 2).
-    constexpr int S = pfbm<M>::S, TT = pfbm<M>::TT, RS = pfbm<M>::RS;
+    constexpr int S = pfbm<M>::S, TT = pfbm<M>::TT, RS = pfbm<M>::RS, D = M / OS;
     extern __shared__ __align__(128) float2 sm[];
-    const int rows = TT + P4 - 1;
+    const int rows = TT + P4 * OS - 1;
     float2* X0 = sm;
-    float2* U = X0 + nbuf * rows * M;
+    float2* U = X0 + nbuf * rows * D;
     float* hT = reinterpret_cast<float*>(U + TT * RS);
     uint64_t* bar = reinterpret_cast<uint64_t*>(hT + P4 * M);
     const int tid = threadIdx.x;
@@ -647,12 +658,12 @@ __global__ void __launch_bounds__(256, (M >= 128 ? 1 : 2))
         sincospif(2.0f * (float)(((tid % S) * c1) % M) / (float)M, &sn, &cs_);
         twr[c1] = make_float2(cs_, sn);
     }
-    const long long nh = (long long)(Ptrue - 1) * M;
+    const long long nh = (long long)(Ptrue - 1) * M + (M - D); // P M - D samples of history
     const long long n_tiles = (n_frames + TT - 1) / TT;
-    const uint32_t tile_bytes = (uint32_t)rows * (uint32_t)M * 8u;
+    const uint32_t tile_bytes = (uint32_t)rows * (uint32_t)D * 8u;
     auto tma_tile = [&](long long t) {
-        const long long g0 = (t * TT - (P4 - 1)) * M;
-        return tma_ok && g0 >= 0 && g0 + (long long)rows * M <= n_in;
+        const long long g0 = (t * TT - (P4 * OS - 1)) * D;
+        return tma_ok && g0 >= 0 && g0 + (long long)rows * D <= n_in;
     };
     __syncthreads();
     pdl_wait();              // programmatic dependent launch: everything above overlapped the previous kernel's tail
@@ -663,28 +674,28 @@ __global__ void __launch_bounds__(256, (M >= 128 ? 1 : 2))
             const long long t = tile + (long long)b * gridDim.x;
             if (t < n_tiles && tma_tile(t)) {
                 mbar_arrive_expect_tx(bar + b, tile_bytes);
-                bulk_copy_g2s(X0 + b * rows * M, x + (t * TT - (P4 - 1)) * M, tile_bytes, bar + b);
+                bulk_copy_g2s(X0 + b * rows * D, x + (t * TT - (P4 * OS - 1)) * D, tile_bytes, bar + b);
             }
         }
     uint32_t phase = 0; // bit b: parity of the next completion of bar[b]
     for (int it = 0; tile < n_tiles; tile += gridDim.x, it++) {
         const long long f0 = tile * TT;
         const int xb = nbuf == 2 ? (it & 1) : 0;
-        float2* X = X0 + xb * rows * M;
+        float2* X = X0 + xb * rows * D;
         if (tma_tile(tile)) {
             mbar_wait(bar + xb, (phase >> xb) & 1u);
             phase ^= 1u << xb;
         } else {
-            const long long g0 = (f0 - (P4 - 1)) * M;
-            for (int i0 = tid; i0 < rows * M; i0 += 256 * 8) {
+            const long long g0 = (f0 - (P4 * OS - 1)) * D;
+            for (int i0 = tid; i0 < rows * D; i0 += 256 * 8) {
                 float2 v[8];
 #pragma unroll
                 for (int u = 0; u < 8; u++)
-                    if (i0 + u * 256 < rows * M)
+                    if (i0 + u * 256 < rows * D)
                         v[u] = pfb_fetch(x, halo, nh, g0 + i0 + u * 256, n_in);
 #pragma unroll
                 for (int u = 0; u < 8; u++)
-                    if (i0 + u * 256 < rows * M)
+                    if (i0 + u * 256 < rows * D)
                         X[i0 + u * 256] = v[u];
             }
             __syncthreads();
@@ -692,7 +703,8 @@ __global__ void __launch_bounds__(256, (M >= 128 ? 1 : 2))
         // ---- branch filters: thread = (branch i, 16 consecutive frames)
         {
             const int i = tid % M, tg = tid / M;
-            const float2* col = X + (M - 1 - i) + (tg * 16) * M;
+            const int a = i / D, b = i % D; // branch i = a D + b: column D-1-b, rows shifted by OS-1-a (see pfb64_kernel)
+            const float2* col = X + (D - 1 - b) + (tg * 16 + OS - 1 - a) * D;
             float2 acc[16];
 #pragma unroll
             for (int j = 0; j < 16; j++)
@@ -703,12 +715,12 @@ __global__ void __launch_bounds__(256, (M >= 128 ? 1 : 2))
                 for (int r = 0; r < P4T; r++)
                     hreg[r] = hT[r * M + i];
 #pragma unroll
-                for (int rho = 0; rho < 16 + P4T - 1; rho++) {
-                    const float2 v = col[rho * M];
+                for (int rho = 0; rho < 16 + (P4T - 1) * OS; rho++) {
+                    const float2 v = col[rho * D];
 #pragma unroll
                     for (int j = 0; j < 16; j++) {
-                        const int r = j + P4T - 1 - rho;
-                        if (r >= 0 && r < P4T)
+                        const int r = P4T - 1 - (rho - j) / OS;
+                        if ((rho - j) % OS == 0 && r >= 0 && r < P4T)
                             acc[j] = __ffma2_rn(v, make_float2(hreg[r], hreg[r]), acc[j]);
                     }
                 }
@@ -716,30 +728,30 @@ __global__ void __launch_bounds__(256, (M >= 128 ? 1 : 2))
                 for (int rc = 0; rc < P4; rc += 4) {
                     const float h0 = hT[(rc + 0) * M + i], h1 = hT[(rc + 1) * M + i];
                     const float h2 = hT[(rc + 2) * M + i], h3 = hT[(rc + 3) * M + i];
-                    const float2* base = col + (P4 - 1 - rc - 3) * M;
-                    float2 w[19];
+                    const float2* base = col + (P4 - 1 - rc - 3) * OS * D;
+                    float2 w[16 + 3 * OS];
 #pragma unroll
-                    for (int q = 0; q < 19; q++)
-                        w[q] = base[q * M];
+                    for (int q = 0; q < 16 + 3 * OS; q++)
+                        w[q] = base[q * D];
 #pragma unroll
                     for (int j = 0; j < 16; j++) {
-                        acc[j] = __ffma2_rn(w[j + 3], make_float2(h0, h0), acc[j]);
-                        acc[j] = __ffma2_rn(w[j + 2], make_float2(h1, h1), acc[j]);
-                        acc[j] = __ffma2_rn(w[j + 1], make_float2(h2, h2), acc[j]);
+                        acc[j] = __ffma2_rn(w[j + 3 * OS], make_float2(h0, h0), acc[j]);
+                        acc[j] = __ffma2_rn(w[j + 2 * OS], make_float2(h1, h1), acc[j]);
+                        acc[j] = __ffma2_rn(w[j + OS], make_float2(h2, h2), acc[j]);
                         acc[j] = __ffma2_rn(w[j], make_float2(h3, h3), acc[j]);
                     }
                 }
             }
 #pragma unroll
-            for (int j = 0; j < 16; j++)
-                U[(tg * 16 + j) * RS + i] = acc[j];
+            for (int j = 0; j < 16; j++) // circular shift of the branches: slot (i - t D) mod M
+                U[(tg * 16 + j) * RS + (OS == 1 ? i : (i - (phase0 + j) * D) & (M - 1))] = acc[j];
         }
         __syncthreads(); // U complete; X fully consumed
         {
             const long long nxt = tile + (long long)nbuf * gridDim.x; // refill the buffer just consumed
             if (tid == 0 && nxt < n_tiles && tma_tile(nxt)) {
                 mbar_arrive_expect_tx(bar + xb, tile_bytes);
-                bulk_copy_g2s(X, x + (nxt * TT - (P4 - 1)) * M, tile_bytes, bar + xb);
+                bulk_copy_g2s(X, x + (nxt * TT - (P4 * OS - 1)) * D, tile_bytes, bar + xb);
             }
         }
         // ---- stage 1: radix 16 over i1 (rows are warp-local: a warp owns 32/S whole frames)
@@ -1094,6 +1106,19 @@ static inline size_t pfbs_rest(int M, int P4)
     return sizeof(float2) * (size_t)M * (TT + TT / 16 + 2) + sizeof(float) * ((size_t)P4 * M + 1) + 32;
 }
 
+// shared memory of the single-pass M = 16 .. 256 kernels (pfb64_kernel, pfbm_kernel) with `nbuf` input tiles of
+// TT + P4 os - 1 rows of D = M / os samples (TT = 4096 / M frames)
+static inline size_t pfb_single_pass_smem(int M, int P4, int os, int nbuf)
+{
+    const int TT = 4096 / M;
+    const size_t xbytes = sizeof(float2) * (size_t)(TT + P4 * os - 1) * (M / os);
+    if (M == 64) {
+        const bool regtaps = P4 == 4 || P4 == 8 || P4 == 12 || P4 == 16 || P4 == 24 || P4 == 32;
+        return nbuf * xbytes + sizeof(float2) * (size_t)PFB64_TT * PFB64_RS + (regtaps ? 0 : sizeof(float) * (size_t)P4 * 64);
+    }
+    return nbuf * xbytes + sizeof(float2) * (size_t)TT * 17 * (M / 16) + sizeof(float) * (size_t)P4 * M + 16;
+}
+
 static inline uint16_t pfb_bf16_rn(float f)
 {
     uint32_t u;
@@ -1125,6 +1150,9 @@ struct b200_pfb {
     int tc_mn = 1;         // pfb64_tc_kernel: branch outputs stored MN-major (16-byte stores), DFT matrix with planar K
     int nbuf = 1;          // input tiles in shared memory (pfbm_kernel)
     int fusedM = 0; // 1: M = 16 / 32 / 128 / 256 on pfbm_kernel; 2: M = 4 / 8 on pfbs_kernel (single pass both)
+    int os = 1;            // oversample rate: one frame per D = M / os input samples
+    int D = 0;
+    int phase = 0;         // frames produced since creation or the last reset, mod os (the branch rotation)
     // generic M >= 16: branch filters -> scratch -> the library's own reverse FFT of length M
     b200_fft* ifft = nullptr;
     float2* d_u = nullptr;    // [chunk_frames][M] branch outputs
@@ -1133,7 +1161,7 @@ struct b200_pfb {
 };
 
 static int pfb_launch(b200_pfb* h, const void* d_halo, const void* d_in, void* d_out,
-                      long long n_in, long long n_frames, cudaStream_t s)
+                      long long n_in, long long n_frames, int phase0, cudaStream_t s)
 {
     if (n_frames <= 0)
         return B200_OK;
@@ -1154,19 +1182,26 @@ static int pfb_launch(b200_pfb* h, const void* d_halo, const void* d_in, void* d
     } else if (h->M == 64) {
         long long tiles = (n_frames + PFB64_TT - 1) / PFB64_TT;
         long long g = tiles < h->grid ? tiles : h->grid;
-#define PFB64_GO(PT)                                                                              \
-    B200_LAUNCH_PDL(pfb64_kernel<PT>, (unsigned)g, 256, h->smem, s, (const float2*)d_in,                  \
+#define PFB64_GO(PT, OS)                                                                          \
+    B200_LAUNCH_PDL((pfb64_kernel<PT, OS>), (unsigned)g, 256, h->smem, s, (const float2*)d_in,            \
                 (const float2*)d_halo, (float2*)d_out, h->d_taps_rm, h->P4, h->P, n_frames, n_in,     \
-                h->ch_begin, h->ch_count, (int)((uintptr_t)d_in % 16 == 0), h->nbuf)
-        switch (h->P4) {
-        case 4: PFB64_GO(4); break;
-        case 8: PFB64_GO(8); break;
-        case 12: PFB64_GO(12); break;
-        case 16: PFB64_GO(16); break;
-        case 24: PFB64_GO(24); break;
-        case 32: PFB64_GO(32); break;
-        default: PFB64_GO(0); break;
+                h->ch_begin, h->ch_count, (int)((uintptr_t)d_in % 16 == 0), h->nbuf, phase0)
+#define PFB64_P(OS)                    \
+    switch (h->P4) {                   \
+    case 4: PFB64_GO(4, OS); break;    \
+    case 8: PFB64_GO(8, OS); break;    \
+    case 12: PFB64_GO(12, OS); break;  \
+    case 16: PFB64_GO(16, OS); break;  \
+    case 24: PFB64_GO(24, OS); break;  \
+    case 32: PFB64_GO(32, OS); break;  \
+    default: PFB64_GO(0, OS); break;   \
+    }
+        switch (h->os) {
+        case 2: PFB64_P(2); break;
+        case 4: PFB64_P(4); break;
+        default: PFB64_P(1); break;
         }
+#undef PFB64_P
 #undef PFB64_GO
     } else if (h->fusedM == 2) {
         const int TT = 4096 / h->M;
@@ -1196,23 +1231,30 @@ static int pfb_launch(b200_pfb* h, const void* d_halo, const void* d_in, void* d
         const int TT = 4096 / h->M;
         long long tiles = (n_frames + TT - 1) / TT;
         long long g = tiles < h->grid ? tiles : h->grid;
-#define PFBM_GO(MM, PT)                                                                               \
-    B200_LAUNCH_PDL((pfbm_kernel<MM, PT>), (unsigned)g, 256, h->smem, s, (const float2*)d_in,             \
+#define PFBM_GO(MM, PT, OS)                                                                           \
+    B200_LAUNCH_PDL((pfbm_kernel<MM, PT, OS>), (unsigned)g, 256, h->smem, s, (const float2*)d_in,         \
                 (const float2*)d_halo, (float2*)d_out, h->d_taps_rm, h->P4, h->P, n_frames, n_in,     \
-                h->ch_begin, h->ch_count, (int)((uintptr_t)d_in % 16 == 0), h->nbuf)
-#define PFBM_P(MM)                         \
+                h->ch_begin, h->ch_count, (int)((uintptr_t)d_in % 16 == 0), h->nbuf, phase0)
+#define PFBM_P(MM, OS)                     \
     switch (h->P4) {                       \
-    case 4: PFBM_GO(MM, 4); break;         \
-    case 8: PFBM_GO(MM, 8); break;         \
-    case 16: PFBM_GO(MM, 16); break;       \
-    default: PFBM_GO(MM, 0); break;        \
+    case 4: PFBM_GO(MM, 4, OS); break;     \
+    case 8: PFBM_GO(MM, 8, OS); break;     \
+    case 16: PFBM_GO(MM, 16, OS); break;   \
+    default: PFBM_GO(MM, 0, OS); break;    \
+    }
+#define PFBM_OS(MM)                        \
+    switch (h->os) {                       \
+    case 2: PFBM_P(MM, 2); break;          \
+    case 4: PFBM_P(MM, 4); break;          \
+    default: PFBM_P(MM, 1); break;         \
     }
         switch (h->M) {
-        case 16: PFBM_P(16); break;
-        case 32: PFBM_P(32); break;
-        case 128: PFBM_P(128); break;
-        default: PFBM_P(256); break;
+        case 16: PFBM_OS(16); break;
+        case 32: PFBM_OS(32); break;
+        case 128: PFBM_OS(128); break;
+        default: PFBM_OS(256); break;
         }
+#undef PFBM_OS
 #undef PFBM_P
 #undef PFBM_GO
     } else if (h->ifft) {
@@ -1274,7 +1316,27 @@ int b200_pfb_create(const b200_pfb_params* p, b200_pfb** out)
     int cb = p->channel_begin, cc = p->channel_count ? p->channel_count : M - p->channel_begin;
     if (cb < 0 || cc < 1 || cb + cc > M)
         return set_err(B200_ERR_ARG, "pfb_create: bad channel slice [%d, %d)", cb, cb + cc);
+    const int os = p->oversample ? p->oversample : 1;
+    if (os != 1 && os != 2 && os != 4)
+        return set_err(B200_ERR_ARG, "pfb_create: oversample %d: need 0 or 1 (critically sampled), 2 or 4", p->oversample);
+    if (os > 1) {
+        // the oversampled bank exists on the single-pass kernels of M = 16 .. 256 only
+        if (M < 16)
+            return set_err(B200_ERR_UNSUPPORTED, "pfb_create: oversample %d needs 16, 32, 64, 128 or 256 channels, not %d", os, M);
+        if (getenv("B200_PFB_TWOPASS"))
+            return set_err(B200_ERR_UNSUPPORTED, "pfb_create: oversample %d runs on the single-pass kernels only, and B200_PFB_TWOPASS is set", os);
+        const int P4 = (P + 3) / 4 * 4;
+        if (pfb_single_pass_smem(M, P4, os, 1) > 220 * 1024) {
+            int pmax = 0;
+            while (pfb_single_pass_smem(M, pmax + 4, os, 1) <= 220 * 1024)
+                pmax += 4;
+            return set_err(B200_ERR_UNSUPPORTED, "pfb_create: taps_per_channel %d too large for oversample %d at M=%d: at most %d", P,
+                           os, M, pmax);
+        }
+    }
     b200_pfb* h = new b200_pfb();
+    h->os = os;
+    h->D = M / os;
     h->M = M;
     h->P = P;
     h->P4 = (P + 3) / 4 * 4;
@@ -1295,34 +1357,45 @@ int b200_pfb_create(const b200_pfb_params* p, b200_pfb** out)
             rm[(size_t)r * M + i] = p->taps[i + r * M];
     PFB_CUDA(cudaMalloc(&h->d_taps_rm, rm.size() * sizeof(float)));
     PFB_CUDA(cudaMemcpy(h->d_taps_rm, rm.data(), rm.size() * sizeof(float), cudaMemcpyHostToDevice));
-    size_t nh = (size_t)(P - 1) * M;
+    size_t nh = (size_t)P * M - h->D;
     for (int i = 0; i < 2; i++) {
         PFB_CUDA(cudaMalloc(&h->d_tail[i], sizeof(float2) * (nh ? nh : 1)));
         PFB_CUDA(cudaMemset(h->d_tail[i], 0, sizeof(float2) * (nh ? nh : 1)));
     }
     if (M == 64) {
-        int rows = PFB64_TT + h->P4 - 1;
+        int rows = PFB64_TT + h->P4 * os - 1;
         const bool regtaps = h->P4 == 4 || h->P4 == 8 || h->P4 == 12 || h->P4 == 16 || h->P4 == 24 || h->P4 == 32;
-        const size_t xb64 = sizeof(float2) * (size_t)rows * 64, u64 = sizeof(float2) * (size_t)PFB64_TT * PFB64_RS;
+        const size_t xb64 = sizeof(float2) * (size_t)rows * h->D, u64 = sizeof(float2) * (size_t)PFB64_TT * PFB64_RS;
         const size_t taps64 = regtaps ? 0 : sizeof(float) * (size_t)h->P4 * 64;
         // second input tile when two CTAs per SM still fit: (233472 - 2 * 1024) / 2 = 115712 bytes per CTA
         // ... and only for 16 taps per channel: the shorter (HBM-bound) filters LOSE with the deeper read prefetch
         // (P = 8: 413 -> 353 GS/s, P = 12: 400 -> 374), P = 16 gains 1.5 % (372.6 -> 378.3)
-        h->nbuf = (regtaps && h->P4 == 16 && 2 * xb64 + u64 <= 115712 && !getenv("B200_PFB_ONEBUF")) ? 2 : 1;
+        // oversampled: B200_PFB_TWOBUF asks for two tiles at any P4 with taps in registers (the A/B of DESIGN.md 4.4e)
+        h->nbuf = (regtaps && (h->P4 == 16 || (os > 1 && getenv("B200_PFB_TWOBUF"))) && 2 * xb64 + u64 <= 115712 &&
+                   !getenv("B200_PFB_ONEBUF")) ? 2 : 1;
         h->smem = h->nbuf * xb64 + u64 + taps64;
         if (h->smem > 220 * 1024) {
             b200_pfb_destroy(h);
             return set_err(B200_ERR_UNSUPPORTED, "pfb_create: taps_per_channel too large for M=64 tile");
         }
-        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
-        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
-        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
-        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
-        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
-        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<24>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
-        PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));
+#define PFB64_ATTR(OS)                                                                                              \
+    PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<0, OS>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));  \
+    PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<4, OS>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));  \
+    PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<8, OS>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR));  \
+    PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<12, OS>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR)); \
+    PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<16, OS>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR)); \
+    PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<24, OS>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR)); \
+    PFB_CUDA(cudaFuncSetAttribute(pfb64_kernel<32, OS>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR))
+        if (os == 2) {
+            PFB64_ATTR(2);
+        } else if (os == 4) {
+            PFB64_ATTR(4);
+        } else {
+            PFB64_ATTR(1);
+        }
+#undef PFB64_ATTR
         h->grid = 2 * sm_count();
-        if (h->P4 <= 16) {
+        if (h->P4 <= 16 && os == 1) { // the tensor-core form exists for the critically sampled bank only
             // tensor-core DFT form: DFT matrix rows m = 2c + part; columns k = 2i + (re | im) for the K-major planes,
             // k = i (re) / 64 + i (im) for the MN-major ones; bf16 hi | lo
             h->tc_mn = 1;
@@ -1369,30 +1442,40 @@ int b200_pfb_create(const b200_pfb_params* p, b200_pfb** out)
 #undef PFBS_ATTR
         h->grid = 2 * sm_count();
     } else if ((M == 16 || M == 32 || M == 128 || M == 256) && !getenv("B200_PFB_TWOPASS") &&
-               sizeof(float2) * ((size_t)(4096 / M + h->P4 - 1) * M + (size_t)(4096 / M) * 17 * (M / 16)) +
-                       sizeof(float) * (size_t)h->P4 * M + 16 <= 220 * 1024) {
+               pfb_single_pass_smem(M, h->P4, os, 1) <= 220 * 1024) {
         h->fusedM = 1;
-        const size_t xbytes = sizeof(float2) * (size_t)(4096 / M + h->P4 - 1) * M;
+        const size_t xbytes = sizeof(float2) * (size_t)(4096 / M + h->P4 * os - 1) * h->D;
         const size_t rest = sizeof(float2) * (size_t)(4096 / M) * 17 * (M / 16) + sizeof(float) * (size_t)h->P4 * M + 16;
         // a second input tile for M >= 128 (one CTA per SM: 321 -> 391 GS/s at M = 128 / P = 8, 335 -> 411 at M = 256 /
         // P = 4).  M = 16 / 32 run two CTAs per SM and LOSE with it (M = 16 / P = 8: 399 -> 345 GS/s; the deeper read
         // prefetch works against the write stream of these HBM-bound kernels), so they keep one.
-        h->nbuf = (M >= 128 && 2 * xbytes + rest <= 227 * 1024 && !getenv("B200_PFB_ONEBUF")) ? 2 : 1;
+        // oversampled: B200_PFB_TWOBUF asks for two tiles at M = 16 / 32 too while two CTAs per SM still fit
+        h->nbuf = ((M >= 128 || (os > 1 && getenv("B200_PFB_TWOBUF") && 2 * xbytes + rest <= 115712)) &&
+                   2 * xbytes + rest <= 227 * 1024 && !getenv("B200_PFB_ONEBUF")) ? 2 : 1;
         h->smem = h->nbuf * xbytes + rest;
-#define PFBM_ATTR(MM)                                                                                          \
-    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR)); \
-    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR)); \
-    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR)); \
-    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR))
+#define PFBM_ATTR(MM, OS)                                                                                          \
+    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 0, OS>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR)); \
+    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 4, OS>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR)); \
+    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 8, OS>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR)); \
+    PFB_CUDA(cudaFuncSetAttribute(pfbm_kernel<MM, 16, OS>, cudaFuncAttributeMaxDynamicSharedMemorySize, PFB_SMEM_ATTR))
+#define PFBM_ATTR_OS(MM)  \
+    if (os == 2) {        \
+        PFBM_ATTR(MM, 2); \
+    } else if (os == 4) { \
+        PFBM_ATTR(MM, 4); \
+    } else {              \
+        PFBM_ATTR(MM, 1); \
+    }
         if (M == 16) {
-            PFBM_ATTR(16);
+            PFBM_ATTR_OS(16);
         } else if (M == 32) {
-            PFBM_ATTR(32);
+            PFBM_ATTR_OS(32);
         } else if (M == 128) {
-            PFBM_ATTR(128);
+            PFBM_ATTR_OS(128);
         } else {
-            PFBM_ATTR(256);
+            PFBM_ATTR_OS(256);
         }
+#undef PFBM_ATTR_OS
 #undef PFBM_ATTR
         h->grid = (M >= 128 ? 1 : 2) * sm_count();
     } else {
@@ -1435,14 +1518,15 @@ int b200_pfb_create(const b200_pfb_params* p, b200_pfb** out)
 int b200_pfb_run(b200_pfb* h, const void* d_in, void* d_out, int64_t n_in_items,
                  int64_t* n_consumed, int64_t* n_produced_vectors, b200_stream_t s)
 {
-    if (!h || n_in_items < 0 || (n_in_items > 0 && !d_in) || (n_in_items >= h->M && !d_out))
+    if (!h || n_in_items < 0 || (n_in_items > 0 && !d_in) || (n_in_items >= h->D && !d_out))
         return set_err(B200_ERR_ARG, "pfb_run: bad argument");
-    long long n_frames = n_in_items / h->M;
-    long long n_cons = n_frames * h->M;
-    int rc = pfb_launch(h, h->d_tail[h->cur], d_in, d_out, n_in_items, n_frames, cs(s));
+    long long n_frames = n_in_items / h->D;
+    long long n_cons = n_frames * h->D;
+    int rc = pfb_launch(h, h->d_tail[h->cur], d_in, d_out, n_in_items, n_frames, h->phase, cs(s));
     if (rc != B200_OK)
         return rc;
-    long long nh = (long long)(h->P - 1) * h->M;
+    h->phase = (int)((h->phase + n_frames) % h->os);
+    long long nh = (long long)h->P * h->M - h->D;
     if (nh > 0 && n_cons > 0) {
         B200_LAUNCH(pfb_tail_kernel, (unsigned)((nh + 255) / 256), 256, 0, cs(s), (const float2*)d_in,
                     h->d_tail[h->cur], h->d_tail[h->cur ^ 1], n_cons, nh);
@@ -1458,10 +1542,10 @@ int b200_pfb_run(b200_pfb* h, const void* d_in, void* d_out, int64_t n_in_items,
 int b200_pfb_run_segment(b200_pfb* h, const void* d_halo, const void* d_in, void* d_out,
                          int64_t n_in_items, int64_t* n_produced_vectors, b200_stream_t s)
 {
-    if (!h || n_in_items < 0 || (n_in_items > 0 && !d_in) || (n_in_items >= h->M && !d_out))
+    if (!h || n_in_items < 0 || (n_in_items > 0 && !d_in) || (n_in_items >= h->D && !d_out))
         return set_err(B200_ERR_ARG, "pfb_run_segment: bad argument");
-    long long n_frames = n_in_items / h->M;
-    int rc = pfb_launch(h, d_halo, d_in, d_out, n_in_items, n_frames, cs(s));
+    long long n_frames = n_in_items / h->D;
+    int rc = pfb_launch(h, d_halo, d_in, d_out, n_in_items, n_frames, 0, cs(s)); // d_in[0] starts frame phase 0
     if (rc == B200_OK && n_produced_vectors)
         *n_produced_vectors = n_frames;
     return rc;
@@ -1473,6 +1557,9 @@ int b200_pfb_set_algorithm(b200_pfb* h, int32_t algorithm)
         return set_err(B200_ERR_ARG, "pfb_set_algorithm: null handle");
     if (algorithm < 0 || algorithm > 2)
         return set_err(B200_ERR_ARG, "pfb_set_algorithm: algorithm must be 0 (auto), 1 (SIMT DFT) or 2 (tensor-core DFT)");
+    if (algorithm == 2 && h->os > 1)
+        return set_err(B200_ERR_UNSUPPORTED, "pfb_set_algorithm: the tensor-core DFT form needs oversample 1 (this handle: %d); "
+                       "oversampled banks run algorithm 0 or 1", h->os);
     if (algorithm == 2 && !h->tc_ok)
         return set_err(B200_ERR_UNSUPPORTED, "pfb_set_algorithm: the tensor-core DFT form needs 64 channels and <= 16 taps per channel");
     h->tc = algorithm == 2 ? 1 : algorithm == 1 ? 0 : (h->tc_ok ? PFB64_TC_DEFAULT : 0);
@@ -1484,6 +1571,14 @@ int b200_pfb_get_algorithm(const b200_pfb* h, int32_t* algorithm)
     if (!h || !algorithm)
         return set_err(B200_ERR_ARG, "pfb_get_algorithm: null argument");
     *algorithm = h->tc ? 2 : 1;
+    return B200_OK;
+}
+
+int b200_pfb_get_oversample(const b200_pfb* h, int32_t* oversample)
+{
+    if (!h || !oversample)
+        return set_err(B200_ERR_ARG, "pfb_get_oversample: null argument");
+    *oversample = h->os;
     return B200_OK;
 }
 
@@ -1502,8 +1597,9 @@ int b200_pfb_reset(b200_pfb* h, b200_stream_t s)
 {
     if (!h)
         return set_err(B200_ERR_ARG, "pfb_reset: null handle");
-    size_t nh = (size_t)(h->P - 1) * h->M;
+    size_t nh = (size_t)h->P * h->M - h->D;
     B200_CUDA(cudaMemsetAsync(h->d_tail[h->cur], 0, sizeof(float2) * (nh ? nh : 1), cs(s)));
+    h->phase = 0;
     return B200_OK;
 }
 

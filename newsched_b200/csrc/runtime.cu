@@ -126,7 +126,7 @@ struct b200_ring {
 
 extern "C" {
 
-int b200_version(void) { return 100; }
+int b200_version(void) { return 101; }
 const char* b200_last_error(void) { return err_buf(); }
 
 int b200_device_count(int* count)
